@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - mode-timesteps/s through WaveformModes.transform (BASELINE.json metric) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n-times T]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n-times T] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): fake_precessing_waveform, ell 2..8 (77 modes), ~1e5 time steps,
 transform(supertranslation with ell<=4, frame_rotation, boost_velocity) -> working band limit 12, 25x25 grid.
@@ -13,6 +13,9 @@ index, no data-path collective): weak scaling; value = total mode-timesteps of a
   e2e   : the public call w.transform(**kwargs) on host numpy arrays: plan construction, H2D, kernels, D2H
   --impl reference : the reference's CPU algorithm (oracle/, a port: the reference itself cannot be
           imported here) on a bounded time-slice of the same waveform, grid points spread over all host cores.
+  --dump-outputs DIR : after the timed steps, rank 0 writes what the last timed step returned (output times and modes,
+          a fixed sample of DUMP_ROWS output times) as float64 .npy files, so that two builds can be compared output
+          for output: the inputs are the same from run to run.
 """
 import argparse
 import json
@@ -120,6 +123,20 @@ class ClockSampler:
                 if val.lower().startswith("active"):
                     reasons.add(nm)
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": smax, "reasons": sorted(reasons), "samples": len(sm)}
+
+
+DUMP_ROWS = 32768   # output times kept by --dump-outputs: 32768 x 77 modes x 16 B = 41 MB, under 64 MB at any --n-times
+
+
+def dump_outputs(out_dir, t, data):
+    """DIR/t.npy: output times; DIR/data.npy: modes as (time, mode, re/im); DIR/rows.npy: which output times these are
+    (all of them when there are at most DUMP_ROWS, else a sorted sample drawn with a fixed seed)."""
+    t, data = t.cpu().numpy(), data.cpu().numpy()
+    n = t.shape[0]
+    rows = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_ROWS), replace=False))
+    np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "t.npy"), t[rows])
+    np.save(os.path.join(out_dir, "data.npy"), np.ascontiguousarray(data[rows]).view(np.float64).reshape(rows.size, *data.shape[1:], 2))
 
 
 def measured_peaks():
@@ -484,7 +501,7 @@ def run_ours(args):
             flush.fill_(1)
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            captured.replay()
+            up, m = captured.replay()
             e1.record()
             torch.cuda.synchronize()
             total_ms += e0.elapsed_time(e1)
@@ -496,6 +513,8 @@ def run_ours(args):
     wall = time.perf_counter() - wall0
     launches = launches_per_step * args.steps      # kernels of ours per step (counted in the eager loop) x timed steps
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, up, m)     # the last timed step's (u', modes'), before anything else runs
 
     # ---- e2e: the public API on host arrays (plan construction + H2D + kernels + D2H inside the timed region)
     # warm-up: the pinned-host caching allocator needs a few calls before result buffers are recycled
@@ -940,7 +959,12 @@ def main():
                     help="transform = configs[1] (the bench line); batch = configs[2]; product = configs[3] (ell<=32 mode products)")
     ap.add_argument("--batch", type=int, default=4096, help="waveforms in the batch workload (all ranks together)")
     ap.add_argument("--no-extras", action="store_true", help="headline line only: skip the configs[2] batch and the time-sharded run")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's output times and modes to DIR/*.npy (float64)")
     args = ap.parse_args()
+    if args.dump_outputs:
+        if args.impl != "ours" or args.workload != "transform":
+            ap.error("--dump-outputs covers the default transform workload of --impl ours")
+        os.makedirs(args.dump_outputs, exist_ok=True)
     claim_stdout()
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3

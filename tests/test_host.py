@@ -2,6 +2,8 @@
 import ctypes
 import os
 import re
+import subprocess
+import sys
 import warnings
 
 import numpy as np
@@ -167,11 +169,15 @@ def test_waveform_shell_history_copy_and_validity():
 
 
 def test_no_cpu_fallback():
-    """Without a CUDA device the operators must fail loudly rather than compute on the CPU."""
+    """Without a CUDA device the operators must fail loudly rather than compute on the CPU.  On a machine with a device
+    this test runs again in a child process that is shown none."""
     import torch
 
     if torch.cuda.is_available():
-        pytest.skip("GPU present")
+        child = subprocess.run([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider", f"{__file__}::test_no_cpu_fallback"],
+                               cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), capture_output=True, text=True)
+        assert child.returncode == 0 and "1 passed" in child.stdout, child.stdout + child.stderr
+        return
     w = sb.sample_waveforms.constant_waveform()
     with pytest.raises(_lib.Scrib200Error):
         w.transform(time_translation=1.0)
