@@ -692,10 +692,18 @@ def test_time_sharded_fluxes_world2():
     assert rel(np.concatenate([r[6] for r in res]), dd) < 1e-10
 
 
-@pytest.mark.parametrize("grid", [dict(n_theta=27, n_phi=31), dict(n_theta=33, n_phi=25), dict(n_theta=26, n_phi=26, ell_max=5)])
+@pytest.mark.parametrize("grid", [dict(n_theta=27, n_phi=31), dict(n_theta=33, n_phi=25), dict(n_theta=26, n_phi=26, ell_max=5),
+                                  dict(ell_max=9), dict(ell_max=10), dict(ell_max=12), dict(n_theta=67, n_phi=19),
+                                  dict(n_theta=19, n_phi=19, ell_max=9), dict(n_theta=31, n_phi=31, ell_max=15)])
 def test_transform_on_user_chosen_grids(grid):
     """`n_theta`, `n_phi` and the output `ell_max` are user keywords (scri/waveform_grid.py:97-110, 627): non-square and
-    oversampled grids take the general analysis path (quadrature tables and tile sizes follow the grid)."""
+    oversampled grids take the general analysis path (quadrature tables and tile sizes follow the grid).  With the
+    supertranslation of BMS the default grid is 25 x 25; the output band limits 9 .. 12 on it and the grids added with them
+    run the non-aliased tiled analysis at time tiles 4 and 2, the aliased one at 2 (67 x 19, also the spline remap's
+    two-step time tile), the persistent tensor-core kernel with two m-blocks (19 x 19, ell_max 9) and the time-major fused
+    kernel (31 x 31, ell_max 15), all through the oracle comparison.  ell_max = 15 needs the larger grid: on 25 rings the
+    quadrature integrand reaches past n_theta - 2, where this quadrature and the oracle's torus extension alias
+    differently (2e-12 apart even in long double)."""
     t, data = smooth_modes(n_times=300, seed=12)
     kw = dict(BMS, **grid)
     out = modes(t, data).transform(**kw)
