@@ -170,6 +170,37 @@ int scrib200_spline_calculus(const double* t, int64_t n_times, const double* dat
 int scrib200_norm(const double* data, int64_t n_times, int n_modes, double* out, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Time-domain inner products: spline definite integrals over time of products of mode series (scri_b200/csrc/inner.cu).
+ * The not-a-knot spline integral of samples f_i is sum_i w_i f_i; the caller computes the weights w [n_times] on the host
+ * once per (t, t1, t2) (scri_b200/ops.py:spline_integral_weights) and passes them as a DEVICE array.
+ *
+ * scrib200_inner_product replaces the integral of scri/mode_calculations.py:493-534 `inner_product` (quaternion.calculus.
+ * spline_definite_integral of abar * b, conj(abar) * b with apply_conjugate) and of scri/waveform_modes.py:574-656
+ * `WaveformModes.inner_product` (sum over modes of conj(a) b, then the same integral):
+ *   a, b    complex128 rows of pitch lda / ldb complex elements; the operands are columns [a_col0, a_col0 + n_cols) and
+ *           [b_col0, b_col0 + n_cols) of them (an ell-clipped view needs no copy)
+ *   n_batch independent products, operand z at a + z a_batch_stride (complex elements; 0 broadcasts one operand)
+ *   conjugate: f(a) = conj(a) (1) or a (0)
+ *   per_column = 0: out [n_batch] complex128, out[z] = sum_i w_i sum_c f(a_ic) b_ic
+ *   per_column = 1: out [n_batch, n_cols] complex128, out[z, c] = sum_i w_i f(a_ic) b_ic
+ *   workspace: scrib200_inner_product_workspace_bytes(n_times, n_cols, n_batch).  Fixed-order reduction, no atomics.
+ *
+ * scrib200_inner_product_matrix: G[p, q] = sum_i w_i sum_m conj(A[p, i, m]) B[q, i, m], the WaveformModes.inner_product of
+ * every pair of two waveform batches (no reference counterpart: the reference computes one pair per call).
+ *   A [P, n_times, n_cols], B [Q, n_times, n_cols] complex128, waveform p at A + p a_stride (complex elements, rows
+ *   contiguous); G [P, Q] complex128; workspace: scrib200_inner_product_matrix_workspace_bytes(P, Q, n_times, n_cols).
+ *   P == 1 or Q == 1 runs the streaming kernel of scrib200_inner_product; otherwise the FP64 tensor-core (DMMA) GEMM with
+ *   K = n_times n_cols split across CTAs and the splits summed in a fixed order.  n_times n_cols < 2^31. */
+size_t scrib200_inner_product_workspace_bytes(int64_t n_times, int n_cols, int n_batch);
+int scrib200_inner_product(const double* a, int64_t lda, int a_col0, int64_t a_batch_stride, const double* b, int64_t ldb,
+                           int b_col0, int64_t b_batch_stride, int64_t n_times, int n_cols, int n_batch, const double* w,
+                           int conjugate, int per_column, double* out, void* workspace, size_t workspace_bytes, void* stream);
+size_t scrib200_inner_product_matrix_workspace_bytes(int P, int Q, int64_t n_times, int n_cols);
+int scrib200_inner_product_matrix(const double* A, int P, int64_t a_stride, const double* B, int Q, int64_t b_stride,
+                                  int64_t n_times, int n_cols, const double* w, double* G, void* workspace,
+                                  size_t workspace_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * <LL> matrix and <L d/dt> vector in one pass over the modes.
  * Replaces  scri/mode_calculations.py:209-295 `_LLMatrix(data, lm, LL)` and :14-43
  * `_LdtVector(data, datadot, lm, Ldt)`.  datadot/Ldt may both be NULL (LL only).

@@ -71,6 +71,13 @@ SIGNATURES = {
     "scrib200_sparse_expectation_ell": (c_int, [c_vp, c_vp, c_i64, c_int, c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp]),
     "scrib200_sparse_expectation_time": (c_int, [c_vp, c_vp, c_i64, c_int, c_vp, c_int, c_int, c_int, c_vp, c_int, c_vp, c_vp]),
     "scrib200_map2salm": (c_int, [c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_sz, c_vp]),
+    "scrib200_inner_product_workspace_bytes": (c_sz, [c_i64, c_int, c_int]),
+    "scrib200_inner_product": (
+        c_int,
+        [c_vp, c_i64, c_int, c_i64, c_vp, c_i64, c_int, c_i64, c_i64, c_int, c_int, c_vp, c_int, c_int, c_vp, c_vp, c_sz, c_vp],
+    ),
+    "scrib200_inner_product_matrix_workspace_bytes": (c_sz, [c_int, c_int, c_i64, c_int]),
+    "scrib200_inner_product_matrix": (c_int, [c_vp, c_int, c_i64, c_vp, c_int, c_i64, c_i64, c_int, c_vp, c_vp, c_vp, c_sz, c_vp]),
 }
 
 

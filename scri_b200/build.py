@@ -11,7 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(CSRC, "_obj")
 LIB = os.path.join(HERE, "libscrib200.so")
-SOURCES = ["runtime.cu", "rotate.cu", "synth.cu", "spline_tile.cu", "mix.cu", "analysis.cu", "modes.cu", "product.cu", "codec.cu"]
+SOURCES = ["runtime.cu", "rotate.cu", "synth.cu", "spline_tile.cu", "mix.cu", "analysis.cu", "modes.cu", "product.cu", "codec.cu", "inner.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

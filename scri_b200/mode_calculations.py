@@ -139,3 +139,66 @@ def rotor_angular_velocity(R, t):
     R = np.asarray(R, dtype=float)
     Rdot = CubicSpline(t, R).derivative()(t)
     return (2 * Q.qmul(Rdot, Q.qconj(R)))[:, 1:]
+
+
+def inner_product(t, abar, b, axis=None, apply_conjugate=False):
+    """Spline definite integral over t[0]..t[-1] of abar * b (conj(abar) * b with `apply_conjugate`), elementwise - no sum
+    over modes (scri/mode_calculations.py:493-534, quaternion.calculus.spline_definite_integral).
+
+    `axis` is the time axis of the (broadcast) integrand; None takes the first axis whose length is t.size.  The result has
+    the integrand's shape without that axis (a 0-d array for 1-D input); it is complex unless both inputs are real.  Device
+    tensors stay on the device (a tensor result), host arrays give numpy.  The integrand is never formed: the time axis is
+    moved to the front and every remaining element is one column of a weighted streaming sum (csrc/inner.cu)."""
+    _lib.require_cuda()
+    t = np.asarray(ops.to_host(t), dtype=float).ravel()
+    on_device = ops.is_tensor(abar) or ops.is_tensor(b)
+    if on_device:
+        import torch
+
+        x, y = (v if ops.is_tensor(v) else torch.as_tensor(np.asarray(v)) for v in (abar, b))
+        x, y = x.cuda(), y.cuda()
+        x, y = torch.broadcast_tensors(x, y)
+        is_complex = x.is_complex() or y.is_complex()
+    else:
+        x, y = np.broadcast_arrays(np.asarray(abar), np.asarray(b))
+        is_complex = np.iscomplexobj(x) or np.iscomplexobj(y)
+    shape = tuple(x.shape)
+    if axis is None:
+        axes = [i for i, n in enumerate(shape) if n == t.size]
+        if not axes:
+            raise ValueError(f"inner_product: no axis of the integrand (shape {shape}) has the length of t ({t.size})")
+        axis = axes[0]
+    axis = int(axis) % len(shape)
+    if shape[axis] != t.size:
+        raise ValueError(f"inner_product: axis {axis} of the integrand (shape {shape}) does not have the length of t ({t.size})")
+    w = ops.spline_integral_weights_device(t)
+    N = t.size
+    rest = shape[:axis] + shape[axis + 1:]
+    if on_device:
+        xm, ym = (v.movedim(axis, 0).reshape(N, -1) for v in (x, y))
+    else:
+        xm, ym = (np.ascontiguousarray(np.moveaxis(v, axis, 0).reshape(N, -1), dtype=np.complex128) for v in (x, y))
+    if xm.shape[1] == 0:
+        out = np.zeros(rest, dtype=complex if is_complex else float)
+        return torch.from_numpy(out).cuda() if on_device else out
+    out = ops.inner_product(xm, ym, w, conjugate=apply_conjugate, per_column=True)
+    out = out.reshape(rest)
+    return out if is_complex else out.real
+
+
+def inner_product_matrix(t, a, b, t1=None, t2=None):
+    """G [P, Q] complex128 with G[p, q] = the inner product of waveform p of `a` with waveform q of `b` - exactly
+    `WaveformModes.inner_product` of that pair: integral from t1 to t2 (default: the first and last time) of
+    sum_m conj(a[p, :, m]) b[q, :, m] through the not-a-knot cubic spline of the samples `t`.
+
+    Not in scri: a project extension for comparing batches (e.g. the [B, N', n] output of parallel.transform_batch) without
+    bringing them back to the host.  a [P, N, n], b [Q, N, n] (or [N, n] for one waveform): numpy arrays or device tensors;
+    a tensor result for tensor input.  One sum per pair on the FP64 tensor cores (P, Q > 1) or the streaming kernel (a single
+    row or column of G), csrc/inner.cu."""
+    _lib.require_cuda()
+    t = np.asarray(ops.to_host(t), dtype=float).ravel()
+    for name, v in (("a", a), ("b", b)):
+        if tuple(v.shape)[-2] != t.size:
+            raise ValueError(f"inner_product_matrix: {name} of shape {tuple(v.shape)} does not have {t.size} time samples on axis -2")
+    w = ops.spline_integral_weights_device(t, t1, t2)
+    return ops.inner_product_matrix(a, b, w)

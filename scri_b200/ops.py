@@ -973,3 +973,171 @@ def sparse_expectation(a, b, matrices):
             "sparse_expectation",
         )
     return out if is_tensor(a) else to_host(out)
+
+
+# ---------------------------------------------------------------------------------- inner products (csrc/inner.cu)
+def _bspline_basis(knots, x, span, p):
+    """[len(x), p + 1]: the nonzero degree-p B-splines B_{span-p} .. B_{span} of `knots` at the points x, where
+    knots[span] <= x <= knots[span + 1] (Cox-de Boor, vectorised over the points)."""
+    x = np.asarray(x, dtype=float)
+    span = np.asarray(span)
+    out = np.zeros((x.size, p + 1))
+    out[:, 0] = 1.0
+    left = np.empty((x.size, p + 1))
+    right = np.empty((x.size, p + 1))
+    for j in range(1, p + 1):
+        left[:, j] = x - knots[span + 1 - j]
+        right[:, j] = knots[span + j] - x
+        saved = np.zeros(x.size)
+        for r in range(j):
+            temp = out[:, r] / (right[:, r + 1] + left[:, j - r])
+            out[:, r] = saved + right[:, r + 1] * temp
+            saved = left[:, j - r] * temp
+        out[:, j] = saved
+    return out
+
+
+def spline_integral_weights(t, t1=None, t2=None):
+    """w [N] float64 with  sum_i w_i f_i = InterpolatedUnivariateSpline(t, f, k=3).integral(t1, t2)  for every f.
+
+    The spline is FITPACK's interpolating cubic (s = 0) on the knots [t0]*4 + t[2:N-2] + [t_{N-1}]*4, i.e. the not-a-knot
+    interpolant: f = M c with the collocation matrix M[i, j] = B_j(t_i), so the integral is beta . M^-1 f with
+    beta_j = integral of B_j over [t1, t2] clipped to [t0, t_{N-1}] (the spline counts as zero outside), and w = M^-T beta.
+    beta comes from the antiderivative of a cubic B-spline, (k_{j+4} - k_j)/4 times the sum of the degree-4 B-splines
+    from j+1 on (knots extended by one at each end); t1 > t2 gives the negative of the integral over [t2, t1].  O(N)
+    host work: two points of degree-4 basis, the banded collocation matrix and one banded solve.  Defaults: t1 = t[0],
+    t2 = t[-1] (quaternion.calculus.spline_definite_integral, used by scri/mode_calculations.py:534)."""
+    from scipy.linalg import solve_banded
+
+    t = np.ascontiguousarray(t, dtype=np.float64)
+    N = t.size
+    if t.ndim != 1 or N < 4:
+        raise ValueError(f"the cubic spline integral needs at least 4 samples; got t of shape {t.shape}")
+    t1 = t[0] if t1 is None else float(t1)
+    t2 = t[-1] if t2 is None else float(t2)
+    sign = 1.0
+    lo, hi = t1, t2
+    if lo > hi:
+        lo, hi, sign = hi, lo, -1.0
+    lo = min(max(lo, t[0]), t[-1])
+    hi = min(max(hi, t[0]), t[-1])
+    if not lo < hi:
+        return np.zeros(N)
+    k = np.concatenate([np.full(4, t[0]), t[2 : N - 2], np.full(4, t[-1])])        # N + 4 knots, N cubic B-splines
+    e = np.concatenate([[t[0]], k, [t[-1]]])                                       # N + 6 knots, N + 1 quartic ones
+
+    def tail_sums(x):
+        # S[m] = sum_{i >= m} E_i(x) for m = 0 .. N + 1 (partition of unity: 1 left of the nonzero window, 0 right of it)
+        s = int(min(max(np.searchsorted(e, x, side="right") - 1, 4), N))
+        vals = _bspline_basis(e, np.array([x]), np.array([s]), 4)[0]
+        S = np.zeros(N + 2)
+        S[: s - 4 + 1] = 1.0
+        for m in range(s - 3, s + 1):
+            S[m] = vals[m - (s - 4):].sum()
+        return S
+
+    c = (k[4:] - k[:N]) / 4.0
+    beta = c * (tail_sums(hi)[1 : N + 1] - tail_sums(lo)[1 : N + 1])
+    # collocation matrix M [N, N] with 2 bands on each side (3 kept for the last row, whose span is the last interval)
+    span = np.clip(np.searchsorted(k, t, side="right") - 1, 3, N - 1)
+    vals = _bspline_basis(k, t, span, 3)                                            # M[i, span_i - 3 + r]
+    L = U = 3
+    ab = np.zeros((L + U + 1, N))                                                   # banded form of M^T
+    rows = np.arange(N)
+    for r in range(4):
+        j = span - 3 + r
+        ab[U + j - rows, rows] = vals[:, r]                                         # M^T[j, i] = M[i, j]
+    return sign * solve_banded((L, U), ab, beta)
+
+
+_weights_cache = {}
+
+
+def spline_integral_weights_device(t, t1=None, t2=None):
+    """`spline_integral_weights` as a device tensor, cached per (t, t1, t2) on the current device."""
+    torch = _torch()
+    t = np.ascontiguousarray(to_host(t), dtype=np.float64)
+    key = (t.tobytes(), None if t1 is None else float(t1), None if t2 is None else float(t2), torch.cuda.current_device())
+    w = _weights_cache.get(key)
+    if w is None:
+        if len(_weights_cache) > 16:
+            _weights_cache.clear()
+        w = _weights_cache[key] = torch.from_numpy(spline_integral_weights(t, t1, t2)).cuda()
+    return w
+
+
+def _complex_device(x):
+    """complex128 CUDA tensor of a host array or a tensor of any dtype."""
+    torch = _torch()
+    d = to_device(x, np.complex128)
+    return d if d.dtype == torch.complex128 else d.to(torch.complex128)
+
+
+def inner_product(a, b, w, conjugate=True, per_column=False, a_cols=None, b_cols=None):
+    """Weighted sums over time of products of two complex series [N, pitch] (scrib200_inner_product):
+    sum_i w_i sum_c f(a_ic) b_ic (a complex scalar tensor / numpy complex) or, with `per_column`, [n] per column;
+    f = conj with `conjugate`.  `a_cols` / `b_cols` = (first column, number of columns) select a window of the rows
+    (default: all columns); `w` [N] float64 (device tensor or host array)."""
+    lib = _lib.load()
+    torch = _torch()
+    ad = _complex_device(a)
+    bd = ad if b is a else _complex_device(b)
+    if ad.dim() != 2 or bd.dim() != 2 or ad.shape[0] != bd.shape[0]:
+        raise ValueError(f"inner_product: operands must be [N, n] with one N; got {tuple(ad.shape)} and {tuple(bd.shape)}")
+    ad, bd = ad.contiguous(), bd.contiguous()
+    N = ad.shape[0]
+    a0, n = a_cols if a_cols is not None else (0, ad.shape[1])
+    b0, nb = b_cols if b_cols is not None else (0, bd.shape[1])
+    if n != nb:
+        raise ValueError(f"inner_product: column windows of {n} and {nb} columns")
+    wd = to_device(w, np.float64)
+    if wd.shape != (N,):
+        raise ValueError(f"inner_product: weights of shape {tuple(wd.shape)} for {N} samples")
+    out = torch.empty(n if per_column else 1, dtype=torch.complex128, device="cuda")
+    ws = torch.empty(max(16, lib.scrib200_inner_product_workspace_bytes(N, n, 1)), dtype=torch.uint8, device="cuda")
+    _lib.check(
+        lib.scrib200_inner_product(_lib.ptr(ad), ad.shape[1], int(a0), 0, _lib.ptr(bd), bd.shape[1], int(b0), 0, N, int(n), 1,
+                                   _lib.ptr(wd), int(bool(conjugate)), int(bool(per_column)), _lib.ptr(out), _lib.ptr(ws),
+                                   ws.numel(), _lib.stream_ptr()),
+        "inner_product",
+    )
+    if not per_column:
+        out = out[0]
+    if is_tensor(a) or is_tensor(b):
+        return out
+    return to_host(out) if per_column else complex(out.item())
+
+
+def _batch_operand(x):
+    """[P, N, n] complex128 device tensor whose rows are contiguous within each waveform, and its waveform stride."""
+    d = _complex_device(x)
+    if d.dim() == 2:
+        d = d.unsqueeze(0)
+    if d.dim() != 3:
+        raise ValueError(f"inner_product_matrix: operands must be [P, N, n]; got shape {tuple(d.shape)}")
+    if d.stride(2) != 1 or d.stride(1) != d.shape[2] or d.stride(0) < d.shape[1] * d.shape[2]:
+        d = d.contiguous()
+    return d, d.stride(0)
+
+
+def inner_product_matrix(A, B, w):
+    """G [P, Q] complex128: G[p, q] = sum_i w_i sum_m conj(A[p, i, m]) B[q, i, m] (scrib200_inner_product_matrix)."""
+    lib = _lib.load()
+    torch = _torch()
+    Ad, sa = _batch_operand(A)
+    Bd, sb = (Ad, sa) if B is A else _batch_operand(B)
+    P, N, n = Ad.shape
+    Q = Bd.shape[0]
+    if Bd.shape[1:] != (N, n):
+        raise ValueError(f"inner_product_matrix: waveforms of shape {tuple(Ad.shape[1:])} and {tuple(Bd.shape[1:])}")
+    wd = to_device(w, np.float64)
+    if wd.shape != (N,):
+        raise ValueError(f"inner_product_matrix: weights of shape {tuple(wd.shape)} for {N} samples")
+    G = torch.empty((P, Q), dtype=torch.complex128, device="cuda")
+    ws = torch.empty(max(16, lib.scrib200_inner_product_matrix_workspace_bytes(P, Q, N, n)), dtype=torch.uint8, device="cuda")
+    _lib.check(
+        lib.scrib200_inner_product_matrix(_lib.ptr(Ad), P, sa, _lib.ptr(Bd), Q, sb, N, n, _lib.ptr(wd), _lib.ptr(G), _lib.ptr(ws),
+                                          ws.numel(), _lib.stream_ptr()),
+        "inner_product_matrix",
+    )
+    return G if (is_tensor(A) or is_tensor(B)) else to_host(G)

@@ -164,6 +164,47 @@ class WaveformModes(WaveformBase):
         self.data = ops.conjugate_pairs(self.data, self.ell_min, self.ell_max, inverse=True)
         self._append_history(f"{self}.convert_from_conjugate_pairs()")
 
+    def inner_product(self, b, t1=None, t2=None, allow_LM_differ=False, allow_times_differ=False):
+        """<self, b> = integral from t1 to t2 of sum over modes of conj(self) b, through the not-a-knot cubic spline in time: a
+        complex scalar (scri/waveform_modes.py:574-656).  Defaults: t1, t2 = the first and last time.
+
+        The checks are those of flux.matrix_expectation_value: spin weights must match; ell ranges must match unless
+        `allow_LM_differ`, which restricts both to the common range; times must match unless `allow_times_differ`, which
+        interpolates both onto `flux.intersection` of the two axes.  On a common time axis the common ell range is a
+        column window of each operand (no copy).  One streaming pass on the GPU (csrc/inner.cu)."""
+        from . import _lib, ops
+        from .flux import intersection
+
+        if self.spin_weight != b.spin_weight:
+            raise ValueError("Spin weights must match in inner_product")
+        ell_min, ell_max = self.ell_min, self.ell_max
+        clip = False
+        if (self.ell_min != b.ell_min) or (self.ell_max != b.ell_max):
+            if not allow_LM_differ:
+                raise ValueError("ell_min and ell_max must match in inner_product (use allow_LM_differ=True to override)")
+            ell_min, ell_max = max(self.ell_min, b.ell_min), min(self.ell_max, b.ell_max)
+            if ell_min >= ell_max + 1:
+                raise ValueError("Intersection of (ell,m) modes is empty.  Assuming this is not desired.")
+            clip = True
+        t_clip = None
+        if not np.array_equal(self.t, b.t):
+            if not allow_times_differ:
+                raise ValueError("Time samples must match in inner_product (use allow_times_differ=True to override)")
+            t_clip = intersection(self.t, b.t)
+        _lib.require_cuda()
+        times, A, B = self.t, self, b
+        n = _sf.LM_total_size(ell_min, ell_max)
+        a_cols = (ell_min**2 - A.ell_min**2, n)
+        b_cols = (ell_min**2 - B.ell_min**2, n)
+        if t_clip is not None:
+            if clip:
+                A, B = A[:, ell_min : ell_max + 1], B[:, ell_min : ell_max + 1]
+                a_cols = b_cols = (0, n)
+            times = t_clip
+            A, B = A.interpolate(t_clip), B.interpolate(t_clip)
+        w = ops.spline_integral_weights_device(times, t1, t2)
+        return ops.inner_product(A.data, B.data, w, conjugate=True, a_cols=a_cols, b_cols=b_cols)
+
     def transform(self, **kwargs):
         """Apply a BMS transformation; returns a new WaveformModes (scri/waveform_modes.py:705-719).
 
