@@ -279,6 +279,15 @@ int scrib200_weyl_mix(const double* const* fields, const double* coef, int n_fie
                       int G, const double* alpha, const double* A, const double* C, const double* scale,
                       const double* offset, double* out, void* stream);
 
+/* The same mix over a batch of n_series series that share the time axis and the transformation (TransformPlan.run_batch
+ * for psi0..psi3, whose companion fields come per waveform): fields[q] and out are [n_series * n_times, G] complex128,
+ * the series stacked along time, and row r takes t[r mod n_times].  Every element takes the operations of
+ * scrib200_weyl_mix in the same order, so a batch equals its series mixed one at a time, bit for bit.  Any row count
+ * launches (64-bit indices; series and slabs of rows stride over the grid); fields[0] may alias out. */
+int scrib200_weyl_mix_series(const double* const* fields, const double* coef, int n_fields, const double* t,
+                             int64_t n_times, int64_t n_series, int G, const double* alpha, const double* A,
+                             const double* C, const double* scale, const double* offset, double* out, void* stream);
+
 /* The packed real operand `Bmat` of scrib200_swsh_synthesize built on the device from the rotor grid:
  * Y[g, (l,m)] = (-1)^s sqrt((2l+1)/4pi) D^l_{m,-s}(R_g) - replaces sf.SWSH_grid(R_j_k, s, ell_max)
  * (scri/waveform_grid.py:470-471) and the host-side packing.

@@ -22,6 +22,7 @@ SIGNATURES = {
     "scrib200_last_error": (ctypes.c_char_p, []),
     "scrib200_launch_count": (c_i64, []),
     "scrib200_weyl_mix": (c_int, [c_vp, c_vp, c_int, c_vp, c_i64, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "scrib200_weyl_mix_series": (c_int, [c_vp, c_vp, c_int, c_vp, c_i64, c_i64, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "scrib200_swsh_pack": (c_int, [c_vp, c_int, c_int, c_int, c_int, c_vp, c_vp, c_int, c_vp, c_int, c_int, c_vp]),
     "scrib200_grid_product": (c_int, [c_vp, c_vp, c_vp, c_i64, c_vp]),
     "scrib200_modes_product_max_shared_bytes": (c_sz, []),

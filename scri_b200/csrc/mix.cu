@@ -7,6 +7,9 @@
 //     z[i, g]   = (t[i] - alpha[g]) * A[g] - C[g]                                    (complex A, C; Q <= 4)
 // evaluated by Horner's rule from the highest field.  HBM-bound: (Q+1) reads + 1 write of 16 bytes per element; one
 // thread owns one grid point (its constants stay in registers) and walks a slab of time steps, lanes along g.
+// weyl_mix_series_kernel (scrib200_weyl_mix_series) does the same over a batch of series that share the time axis, row r
+// taking t[r mod n_times]: the batched, graph-captured and time-sharded transforms of psi0..psi3 (TransformPlan.run_batch,
+// capture, parallel.sharded_transform) mix through it, and so does TransformPlan.run with n_series = 1.
 #include "common.cuh"
 
 namespace scrib200 {
@@ -15,6 +18,29 @@ struct MixFields {
     const double2* F[5];
     double c[5];
 };
+
+// One element of the mix, called by both kernels.  Every rounding is spelled out (fma, __dmul_rn, __dsub_rn), so that
+// neither nvcc nor ptxas is free to contract a product into an FMA differently in the two kernels: a batch mixed by
+// weyl_mix_series_kernel equals its series mixed one at a time by weyl_mix_kernel, bit for bit.  (The same expression
+// written as `dt * a.x - c.x` and `cmul(acc, z)` was contracted one way inline in weyl_mix_kernel and another way once
+// moved into a shared function.)  The contractions are those nvcc chose for the original inline body of weyl_mix_kernel:
+//     z = fma(a, dt, -c),   acc z = (fma(z.x, acc.x, -(z.y acc.y)), fma(z.x, acc.y, z.y acc.x)),
+// and, for a single field, out = scale fma(c_0, F_0, -offset).
+__device__ __forceinline__ double2 weyl_mix_element(const MixFields& f, int nq, int64_t e, double ti, double al, double2 a,
+                                                    double2 c, double sc, double2 off) {
+    const double2 top = f.F[nq - 1][e];
+    if (nq == 1) return make_double2(__dmul_rn(sc, fma(f.c[0], top.x, -off.x)), __dmul_rn(sc, fma(f.c[0], top.y, -off.y)));
+    const double dt = __dsub_rn(ti, al);
+    const double2 z = make_double2(fma(a.x, dt, -c.x), fma(a.y, dt, -c.y));
+    double2 acc = make_double2(__dmul_rn(f.c[nq - 1], top.x), __dmul_rn(f.c[nq - 1], top.y));
+    for (int q = nq - 2; q >= 0; --q) {
+        acc = make_double2(fma(z.x, acc.x, -__dmul_rn(z.y, acc.y)), fma(z.x, acc.y, __dmul_rn(z.y, acc.x)));
+        const double2 v = f.F[q][e];
+        acc.x = fma(f.c[q], v.x, acc.x);
+        acc.y = fma(f.c[q], v.y, acc.y);
+    }
+    return make_double2(__dmul_rn(sc, __dsub_rn(acc.x, off.x)), __dmul_rn(sc, __dsub_rn(acc.y, off.y)));
+}
 
 __global__ void __launch_bounds__(128)
 weyl_mix_kernel(MixFields f, int nq, const double* __restrict__ t, int64_t N, int G, const double* __restrict__ alpha,
@@ -28,17 +54,33 @@ weyl_mix_kernel(MixFields f, int nq, const double* __restrict__ t, int64_t N, in
     const int64_t i0 = (int64_t)blockIdx.y * rows_per_cta;
     const int64_t i1 = (i0 + rows_per_cta < N) ? i0 + rows_per_cta : N;
     for (int64_t i = i0; i < i1; ++i) {
-        const double dt = t[i] - al;
-        const double2 z = make_double2(dt * a.x - c.x, dt * a.y - c.y);
         const int64_t e = i * G + g;
-        double2 acc = cscale(f.c[nq - 1], f.F[nq - 1][e]);
-        for (int q = nq - 2; q >= 0; --q) {
-            acc = cmul(acc, z);
-            const double2 v = f.F[q][e];
-            acc.x = fma(f.c[q], v.x, acc.x);
-            acc.y = fma(f.c[q], v.y, acc.y);
+        out[e] = weyl_mix_element(f, nq, e, t[i], al, a, c, sc, off);
+    }
+}
+
+// Slab k of series s covers rows s * n_times + [k * rows_per_cta, (k + 1) * rows_per_cta) and reads t from row k * rows_per_cta
+// on.  Slabs stride over gridDim.y and series over gridDim.z (each capped at 65535), so any row count launches.  `out` may
+// alias field 0: every element is read and written by the same thread, reads first.
+__global__ void __launch_bounds__(128)
+weyl_mix_series_kernel(MixFields f, int nq, const double* __restrict__ t, int64_t n_times, int64_t n_series, int G,
+                       const double* __restrict__ alpha, const double2* __restrict__ A, const double2* __restrict__ C,
+                       const double* __restrict__ scale, const double2* __restrict__ offset, double2* out, int rows_per_cta) {
+    const int g = blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= G) return;
+    const double al = alpha[g], sc = scale[g];
+    const double2 a = A[g], c = C[g];
+    const double2 off = offset ? offset[g] : make_double2(0.0, 0.0);
+    const int64_t n_slabs = (n_times + rows_per_cta - 1) / rows_per_cta;
+    for (int64_t s = blockIdx.z; s < n_series; s += gridDim.z) {
+        for (int64_t k = blockIdx.y; k < n_slabs; k += gridDim.y) {
+            const int64_t i0 = k * rows_per_cta;
+            const int64_t i1 = (i0 + rows_per_cta < n_times) ? i0 + rows_per_cta : n_times;
+            for (int64_t i = i0; i < i1; ++i) {
+                const int64_t e = (s * n_times + i) * G + g;
+                out[e] = weyl_mix_element(f, nq, e, t[i], al, a, c, sc, off);
+            }
         }
-        out[e] = make_double2(sc * (acc.x - off.x), sc * (acc.y - off.y));
     }
 }
 
@@ -86,6 +128,36 @@ extern "C" int scrib200_weyl_mix(const double* const* fields, const double* coef
         f, n_fields, t, n_times, G, alpha, reinterpret_cast<const double2*>(A), reinterpret_cast<const double2*>(C), scale,
         reinterpret_cast<const double2*>(offset), reinterpret_cast<double2*>(out), rows);
     SCRIB200_CHECK_LAUNCH("weyl_mix");
+    return SCRIB200_OK;
+}
+
+extern "C" int scrib200_weyl_mix_series(const double* const* fields, const double* coef, int n_fields, const double* t,
+                                        int64_t n_times, int64_t n_series, int G, const double* alpha, const double* A,
+                                        const double* C, const double* scale, const double* offset, double* out, void* stream) {
+    using namespace scrib200;
+    SCRIB200_REQUIRE(fields && coef && t && alpha && A && C && scale && out, "weyl_mix_series: null pointer");
+    SCRIB200_REQUIRE(n_fields >= 1 && n_fields <= 5, "weyl_mix_series: n_fields=%d must be 1..5", n_fields);
+    SCRIB200_REQUIRE(G > 0, "weyl_mix_series: G=%d", G);
+    SCRIB200_REQUIRE(n_times >= 0 && n_series >= 0, "weyl_mix_series: n_times=%lld n_series=%lld", (long long)n_times,
+                     (long long)n_series);
+    if (n_times == 0 || n_series == 0) return SCRIB200_OK;
+    SCRIB200_REQUIRE(n_times <= INT64_MAX / n_series / G, "weyl_mix_series: %lld x %lld rows of %d points overflow 64-bit indices",
+                     (long long)n_series, (long long)n_times, G);
+    MixFields f;
+    for (int q = 0; q < 5; ++q) {
+        f.F[q] = (q < n_fields) ? reinterpret_cast<const double2*>(fields[q]) : nullptr;
+        f.c[q] = (q < n_fields) ? coef[q] : 0.0;
+        SCRIB200_REQUIRE(q >= n_fields || (fields[q] && aligned16(fields[q])), "weyl_mix_series: field %d is null or misaligned", q);
+    }
+    SCRIB200_REQUIRE(aligned16(A) && aligned16(C) && aligned16(out) && aligned16(offset),
+                     "weyl_mix_series: pointers must be 16-byte aligned");
+    const int rows = 64;
+    const int64_t slabs = (n_times + rows - 1) / rows;
+    dim3 grid((G + 127) / 128, (unsigned)(slabs < 65535 ? slabs : 65535), (unsigned)(n_series < 65535 ? n_series : 65535));
+    weyl_mix_series_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(
+        f, n_fields, t, n_times, n_series, G, alpha, reinterpret_cast<const double2*>(A), reinterpret_cast<const double2*>(C),
+        scale, reinterpret_cast<const double2*>(offset), reinterpret_cast<double2*>(out), rows);
+    SCRIB200_CHECK_LAUNCH("weyl_mix_series");
     return SCRIB200_OK;
 }
 

@@ -142,37 +142,64 @@ def sharded_fluxes(t_local, data_local, ell_min, ell_max, halo=HALO, group=None)
     return edot, pdot, jdot
 
 
-def transform_batch(plan, t, data_batch):
-    """Run one TransformPlan over a local shard `data_batch[B_local, N, n]` (device tensors): (u', modes'[B_local, N', n'])."""
-    return plan.run_batch(t, data_batch)
+def transform_batch(plan, t, data_batch, companions=None):
+    """Run one TransformPlan over a local shard `data_batch[B_local, N, n]` (device tensors): (u', modes'[B_local, N', n']).
+    psi0..psi3 take their companion fields as [B_local, N, n_q] device tensors ordered psi(n+1)..psi4 (plan.run_batch)."""
+    return plan.run_batch(t, data_batch, companions=companions)
 
 
-def transform_batch_host(plan, t, data_host, sub_batch=512, out=None):
+def transform_batch_host(plan, t, data_host, sub_batch=None, out=None, companions_host=None):
     """BASELINE configs[2] from host memory: `data_host` [B, N, n_modes] complex128 numpy (this rank's shard of the batch;
     page-locked memory goes up by DMA, anything else through the staging ring) -> (u' [N'] numpy, modes' [B, N', n_out]
     numpy in pinned memory).  Sub-batches are double-buffered on the device: the H2D of sub-batch i+1 and the D2H of
     sub-batch i-1 run on their own streams under the kernels of sub-batch i (plan.run_batch).  `data_host` may also be a
     sequence of such arrays (a shard that lives in several host blocks): they flow through ONE pipeline without draining
-    in between, and `out`, if given, is the matching sequence of result arrays (a list of results is returned)."""
+    in between, and `out`, if given, is the matching sequence of result arrays (a list of results is returned).
+
+    psi0..psi3 need `companions_host`, parallel to `data_host`: for one array, the sequence of Q host arrays
+    [B, N, n_q] ordered psi(n+1)..psi4; for a sequence of blocks, one such sequence per block.  They go up with the
+    sub-batch they belong to, in the same double-buffered pipeline.
+
+    `sub_batch` defaults to 512 waveforms, and to 512 // (Q + 1) for a plan that mixes in Q companions, so that a psi plan
+    needs no more device memory than an h plan.  Per waveform of N samples on G grid points, with n_q modes per field
+    (16-byte complex), an h plan holds two input buffers (2 * 16 N n), the synthesized and the remapped grid (2 * 16 N G)
+    and the modes (16 N' n_out); a psi plan holds 2 * 16 N sum(n_q) of inputs and, while it mixes, Q + 1 grids - on
+    (Q + 1) times fewer waveforms.  At the shape of configs[2] (N = 2048, ell <= 8, G = 625) an h sub-batch of 512 holds
+    2.6 GB of inputs and 21.0 GB of grids; a psi2 sub-batch of 170 (Q = 2) holds 2.7 GB of inputs and at most 10.4 GB of
+    grids."""
     import ctypes
 
     import torch
 
     from . import _lib, ops
 
-    lib = _lib.load()
-    t_d = ops.to_device(t, np.float64)
     single = isinstance(data_host, np.ndarray)
     blocks = [data_host] if single else list(data_host)
+    n_comp = len(plan.mix)
+    if n_comp and companions_host is None:
+        raise ValueError("transform_batch_host of psi0..psi3 needs companions_host (host arrays of psi(n+1)..psi4)")
+    if companions_host is not None and not n_comp:
+        plan._check_companions(companions_host, (), host=True)   # raises: this plan mixes in no companion fields
+    comp_blocks = [[]] * len(blocks)
+    if n_comp:
+        comp_blocks = [companions_host] if single else list(companions_host)
+        if len(comp_blocks) != len(blocks):
+            raise ValueError(f"companions_host has {len(comp_blocks)} blocks for {len(blocks)} blocks of data")
+        comp_blocks = [plan._check_companions(cb, block.shape[:2], host=True) for block, cb in zip(blocks, comp_blocks)]
     outs = [out] if single else (list(out) if out is not None else [None] * len(blocks))
     blocks = [b if (b.dtype == np.complex128 and b.flags.c_contiguous) else np.ascontiguousarray(b, dtype=np.complex128) for b in blocks]
     N, n = blocks[0].shape[1:]
+    if sub_batch is None:
+        sub_batch = 512 // (n_comp + 1)
     sub = max(1, min(int(sub_batch), max(b.shape[0] for b in blocks)))
+    lib = _lib.load()
+    t_d = ops.to_device(t, np.float64)
     cur = torch.cuda.current_stream()
     cin, cout = torch.cuda.Stream(), torch.cuda.Stream()
     prep = plan.prepare(t_d)             # one time axis for the whole batch: its spline tables and retained block, once
     prep.resolve()
     bufs = [torch.empty((sub, N, n), dtype=torch.complex128, device="cuda") for _ in range(2)]
+    cbufs = [[torch.empty((sub, N, mx["n_modes"]), dtype=torch.complex128, device="cuda") for mx in plan.mix] for _ in range(2)]
     free = [None, None]                                   # event: the kernels that read buffer b are done
     row_bytes = N * n * 16
     u_host = None
@@ -189,10 +216,14 @@ def transform_batch_host(plan, t, data_host, sub_batch=512, out=None):
                 cin.wait_stream(cur)
             _lib.check(lib.scrib200_h2d(bufs[b].data_ptr(), block.ctypes.data + b0 * row_bytes, nb * row_bytes,
                                         ctypes.c_void_p(cin.cuda_stream)), "h2d")
+            for c, cbuf in zip(comp_blocks[k], cbufs[b]):
+                c_row = N * c.shape[2] * 16
+                _lib.check(lib.scrib200_h2d(cbuf.data_ptr(), c.ctypes.data + b0 * c_row, nb * c_row, ctypes.c_void_p(cin.cuda_stream)),
+                           "h2d")
             landed = torch.cuda.Event()
             landed.record(cin)
             cur.wait_event(landed)
-            u, m = plan.run_batch(t_d, bufs[b][:nb], prep=prep)
+            u, m = plan.run_batch(t_d, bufs[b][:nb], prep=prep, companions=[cb[:nb] for cb in cbufs[b]] if n_comp else None)
             done = torch.cuda.Event()
             done.record(cur)
             free[b] = done
@@ -233,19 +264,24 @@ def transform_halo(plan, t_first, t_last, dt_min):
     return int(math.ceil(drift / dt_min)) + SPLINE_DECAY_ROWS + 2
 
 
-def sharded_transform(plan, t_local, data_local, halo=None, group=None, timings=None):
+def sharded_transform(plan, t_local, data_local, companions_local=None, halo=None, group=None, timings=None):
     """WaveformModes.transform (scri/waveform_grid.py:331-630) of ONE long series sharded by TIME: every rank holds a
     contiguous block of (t, modes), ranks in time order.  Each rank borrows `halo` input samples from its neighbours
     (point-to-point: the only data-path communication besides the few scalars below), synthesizes the extended block,
     builds the splines of the extended block and evaluates them at the output times of the samples it owns, masked by the
     GLOBAL retained range; the analysis is pointwise in time.  Returns (u'_local, modes'_local); `gather_batch` assembles
     the full series where wanted.  `halo=None` sizes the halo from the transformation (`transform_halo`); a boost needs
-    beta |t| / dt extra samples, and when that exceeds a neighbour's block the call refuses (shard by waveform instead)."""
+    beta |t| / dt extra samples, and when that exceeds a neighbour's block the call refuses (shard by waveform instead).
+
+    psi0..psi3 need `companions_local`: this rank's block of each higher Weyl scalar, [n_local, n_q] device tensors ordered
+    psi(n+1)..psi4.  The same halo is borrowed for each of them, and the extended block is synthesized and mixed with the
+    extended time axis.  The mixing is pointwise in time and the spline acts on the mixed grid, so the halo does not grow."""
     import torch
     import torch.distributed as dist
 
-    if plan.mix:
-        raise NotImplementedError("sharded_transform does not cover psi0..psi3 (their mixing needs the companion fields)")
+    if plan.mix and companions_local is None:
+        raise ValueError("sharded_transform of psi0..psi3 needs companions_local=[psi(n+1), ..., psi4] as device tensors")
+    plan._check_companions(companions_local, (int(data_local.shape[0]),))
     rank, world = dist.get_rank(group), dist.get_world_size(group)
     dev = t_local.device
     n_loc = int(t_local.shape[0])
@@ -277,10 +313,16 @@ def sharded_transform(plan, t_local, data_local, halo=None, group=None, timings=
     mark("halo_begin")
     prev_d, next_d = exchange_halos(data_local, halo, group)
     prev_t, next_t = exchange_halos(t_local, halo, group)
+    c_ext = None
+    if companions_local is not None:
+        c_ext = []
+        for c in companions_local:
+            prev_c, next_c = exchange_halos(c, halo, group)
+            c_ext.append(torch.cat([x for x in (prev_c, c, next_c) if x is not None]))
     mark("halo_end")
     t_ext = torch.cat([x for x in (prev_t, t_local, next_t) if x is not None])
     d_ext = torch.cat([x for x in (prev_d, data_local, next_d) if x is not None])
-    F = plan.synthesize(d_ext)
+    F = plan.synthesize(d_ext, t_ext, companions=c_ext)
     prep = plan.prepare(t_ext)                                              # spline factor table of the extended block
     # output times of the samples this rank owns, masked by the global retained range (waveform_grid.py:564-568)
     if plan.divide_by_gamma:

@@ -478,9 +478,12 @@ class TransformPlan(GridPlan):
                     w_temp = leftover.pop(key)
                     Yt = _sf.SWSH_grid(R, w_temp.spin_weight, w_temp.ell_max)
                     Bt, Kp, Np = pack_synthesis_matrix(Yt, w_temp.ell_min, w_temp.ell_max)
+                    # the layout is what companions passed per call (run(companions=...)) must match; `data` is what
+                    # run and synthesize use without them
                     self.mix.append(dict(
-                        coef=float(comb(5 - self.dataType, 5 - DT)), data=w_temp.data, n_modes=w_temp.data.shape[1], Kpad=Kp,
-                        Ncpad=Np, d_B=torch.from_numpy(Bt).to(self.device),
+                        dataType=DT, spin_weight=int(w_temp.spin_weight), ell_min=int(w_temp.ell_min),
+                        ell_max=int(w_temp.ell_max), coef=float(comb(5 - self.dataType, 5 - DT)), data=w_temp.data,
+                        n_modes=w_temp.data.shape[1], Kpad=Kp, Ncpad=Np, d_B=torch.from_numpy(Bt).to(self.device),
                     ))
             elif self.dataType not in (psi4, hdot, news):
                 warnings.warn(
@@ -574,19 +577,76 @@ class TransformPlan(GridPlan):
                 "swsh_synthesize_3m",
             )
 
-    def synthesize(self, data, t=None, slabs=None):
+    def _check_companions(self, companions, rows, host=False):
+        """Check the companion fields of psi0..psi3 passed to one call: a list or tuple ordered psi(n+1)..psi4, each of
+        shape `rows` + (n_modes_q,) in the layout of the psi*_modes the plan was built with - C-contiguous complex128 device
+        tensors, or with `host` numpy arrays (returned as C-contiguous complex128 arrays).  Returns the list (or None);
+        raises ValueError, and launches nothing."""
+        if companions is None:
+            return None
+        name = DataNames[self.dataType]
+        if not self.mix:
+            raise ValueError(f"companions were passed to a plan for {name}, which mixes in no companion fields")
+        want = ", ".join(DataNames[mx["dataType"]] for mx in self.mix)
+        if not isinstance(companions, (list, tuple)) or len(companions) != len(self.mix):
+            got = f"{len(companions)} fields" if isinstance(companions, (list, tuple)) else f"a {type(companions).__name__}"
+            raise ValueError(f"{name} needs a list of {len(self.mix)} companion fields ordered {want}; got {got}")
+        torch = self.torch
+        index = self.device.index if self.device.index is not None else torch.cuda.current_device()
+        out = []
+        for mx, c in zip(self.mix, companions):
+            shape = tuple(int(r) for r in rows) + (mx["n_modes"],)
+            if host:
+                ok = isinstance(c, np.ndarray) and c.shape == shape and np.can_cast(c.dtype, np.complex128, "same_kind")
+                kind, got = "numpy array", (f"{c.dtype} array of shape {c.shape}" if isinstance(c, np.ndarray) else type(c).__name__)
+            else:
+                ok = (torch.is_tensor(c) and c.is_cuda and c.device.index == index and c.dtype == torch.complex128
+                      and tuple(c.shape) == shape and c.is_contiguous())
+                kind = f"contiguous complex128 tensor on cuda:{index}"
+                got = (f"{c.dtype} tensor of shape {tuple(c.shape)} on {c.device}{'' if c.is_contiguous() else ', not contiguous'}"
+                       if torch.is_tensor(c) else type(c).__name__)
+            if not ok:
+                raise ValueError(
+                    f"{name}: the companion field {DataNames[mx['dataType']]} (ell {mx['ell_min']}..{mx['ell_max']}, "
+                    f"spin weight {mx['spin_weight']}; companions are ordered {want}) must be a {kind} of shape {shape}; "
+                    f"got a {got}")
+            out.append(np.ascontiguousarray(c, dtype=np.complex128) if host else c)
+        return out
+
+    def synthesize(self, data, t=None, slabs=None, companions=None):
         """[N, n_modes] complex128 -> F [N, G] complex128 (waveform_grid.py:475-559).  `t` (device) is needed for
         psi0..psi3 only, whose mixing factor depends on time.  `slabs` = [(row_lo, row_hi, event, flag), ...]: the rows of
         `data` are still arriving from the host slab by slab (ops.to_device_slabs); each slab is synthesized as soon as its
-        event has fired, so the GEMM runs under the rest of the transfer."""
+        event has fired, so the GEMM runs under the rest of the transfer.  `companions` (psi0..psi3): the higher Weyl
+        scalars of this call, [N, n_modes_q] device tensors ordered psi(n+1)..psi4 (`_check_companions`); None uses the
+        psi*_modes the plan was built with, uploaded on every call."""
+        N = data.shape[0]
+        comps = self._check_companions(companions, (N,))
+        if self.mix and t is None:
+            raise ValueError("TransformPlan.synthesize needs the time axis for psi0..psi3")
+        if self.mix and comps is None:
+            from . import ops
+
+            comps = []
+            for mx in self.mix:
+                d = ops.to_device(mx["data"], np.complex128)
+                if d.shape[0] != N:
+                    raise ValueError("psi*_modes must share the time axis of the waveform being transformed")
+                comps.append(d)
+        return self._synthesize(data, t, slabs, comps, 1)
+
+    def _synthesize(self, data, t, slabs, comps, n_series):
+        """Synthesis of `data` [n_series * N, n_modes] (series stacked along time), then for psi0..psi3 the synthesis of each
+        companion [n_series * N, n_modes_q] (the folded kernel, offset 0, scale 1) and one scrib200_weyl_mix_series launch
+        that mixes them into F in place (t [N] serves every series)."""
         import ctypes
 
         torch = self.torch
         lib = _lib.load()
-        N = data.shape[0]
-        F = torch.empty((N, self.G), dtype=torch.complex128, device=self.device)
+        rows = data.shape[0]
+        F = torch.empty((rows, self.G), dtype=torch.complex128, device=self.device)
         cur = torch.cuda.current_stream()
-        for lo, hi, ev, flag in (slabs or [(0, N, None, None)]):
+        for lo, hi, ev, flag in (slabs or [(0, rows, None, None)]):
             if ev is not None:
                 flag.wait()            # the copy thread has recorded the event (waiting on an unrecorded event is a no-op)
                 cur.wait_event(ev)
@@ -595,19 +655,12 @@ class TransformPlan(GridPlan):
             self._synthesize_rows(data[lo:hi], F[lo:hi])
         if not self.mix:
             return F
-        if t is None:
-            raise ValueError("TransformPlan.synthesize needs the time axis for psi0..psi3")
-        from . import ops
-
         fields, coefs = [F], [1.0]
-        for mx in self.mix:
-            d = ops.to_device(mx["data"], np.complex128)
-            if d.shape[0] != N:
-                raise ValueError("psi*_modes must share the time axis of the waveform being transformed")
-            Fq = torch.empty((N, self.G), dtype=torch.complex128, device=self.device)
+        for mx, d in zip(self.mix, comps):
+            Fq = torch.empty((rows, self.G), dtype=torch.complex128, device=self.device)
             _lib.check(
                 lib.scrib200_swsh_synthesize(
-                    _lib.ptr(d), N, mx["n_modes"], _lib.ptr(mx["d_B"]), mx["Kpad"], mx["Ncpad"], _lib.ptr(self.d_zero),
+                    _lib.ptr(d), rows, mx["n_modes"], _lib.ptr(mx["d_B"]), mx["Kpad"], mx["Ncpad"], _lib.ptr(self.d_zero),
                     _lib.ptr(self.d_unit), self.G, _lib.ptr(Fq), _lib.stream_ptr(),
                 ),
                 "swsh_synthesize",
@@ -617,11 +670,11 @@ class TransformPlan(GridPlan):
         ptrs = (ctypes.c_void_p * len(fields))(*[f.data_ptr() for f in fields])
         cf = (ctypes.c_double * len(coefs))(*coefs)
         _lib.check(
-            lib.scrib200_weyl_mix(
-                ptrs, cf, len(fields), _lib.ptr(t), N, self.G, _lib.ptr(self.d_alpha), _lib.ptr(self.d_mixA),
-                _lib.ptr(self.d_mixC), _lib.ptr(self.d_mixscale), None, _lib.ptr(F), _lib.stream_ptr(),
+            lib.scrib200_weyl_mix_series(
+                ptrs, cf, len(fields), _lib.ptr(t), rows // n_series, n_series, self.G, _lib.ptr(self.d_alpha),
+                _lib.ptr(self.d_mixA), _lib.ptr(self.d_mixC), _lib.ptr(self.d_mixscale), None, _lib.ptr(F), _lib.stream_ptr(),
             ),
-            "weyl_mix",
+            "weyl_mix_series",
         )
         return F
 
@@ -790,14 +843,18 @@ class TransformPlan(GridPlan):
             return self._run_streaming(t, data, slabs, t_host, debug_poison=debug_poison, _speculate=False)
         return u_np, host_np
 
-    def run(self, t, data, return_grid=False, t_ends=None, prep=None, slabs=None, host_slabs=0, t_host=None, on_queued=None):
+    def run(self, t, data, return_grid=False, t_ends=None, prep=None, slabs=None, host_slabs=0, t_host=None, on_queued=None,
+            companions=None):
         """Whole path on device tensors: returns (u', modes') or (u', grid' [time-major]).
 
         The only host round trip is the 64-byte `info` read-back (size of the retained block); it travels on a side
         stream while the synthesis kernel runs.  `prep` (from `prepare(t)`) can be reused for waveforms that share
         their time axis.  With `host_slabs` = S > 0 the modes come back as a numpy array in pinned host memory: the output
         times are cut into S slabs, each remapped, analysed and copied out on a copy stream while the next one computes
-        (the end-to-end path of WaveformGrid.transform)."""
+        (the end-to-end path of WaveformGrid.transform).  `companions` (psi0..psi3 only): this waveform's higher Weyl
+        scalars as [N, n_modes_q] complex128 device tensors ordered psi(n+1)..psi4, in the layout of the psi*_modes the plan
+        was built with; None uses those psi*_modes themselves."""
+        self._check_companions(companions, (data.shape[0],))
         if host_slabs and slabs is not None and t_host is not None and prep is None and self.tile and not self.mix and not return_grid:
             streamed = self._run_streaming(t, data, slabs, t_host, on_queued=on_queued)
             if streamed is not None:
@@ -805,7 +862,7 @@ class TransformPlan(GridPlan):
         cur = self.torch.cuda.current_stream()
         ready = self.torch.cuda.Event()
         ready.record(cur)
-        F = self.synthesize(data, t, slabs)     # queued first: the GPU is busy while the host launches the preparation
+        F = self.synthesize(data, t, slabs, companions)     # queued first: the GPU is busy while the host launches the preparation
         mine = prep is None
         for attempt in range(2):
             if mine:
@@ -834,19 +891,20 @@ class CapturedTransform:
     CUDA graph: `replay()` re-runs it on the CURRENT contents of the `t` and `data` tensors it was captured with, in one
     launch - the host is then no longer on the critical path of a step (eager, a step is ~25 launches and a few dozen
     tensor allocations; a busy or throttled host shows up as gaps between the kernels).  The retained block found when the
-    graph was captured is baked into it; `verify()` checks it against what the last replay found."""
+    graph was captured is baked into it; `verify()` checks it against what the last replay found.  For psi0..psi3 the
+    graph also reads the companion tensors it was captured with (`companions`), at their contents of each replay."""
 
-    def __init__(self, plan, t, data):
+    def __init__(self, plan, t, data, companions=None):
         torch = plan.torch
-        self.plan, self.t, self.data = plan, t, data
-        plan.run(t, data)                                   # warms every cache the capture must not touch (memo, workspace, pinned pool)
+        self.plan, self.t, self.data, self.companions = plan, t, data, companions
+        plan.run(t, data, companions=companions)            # warms every cache the capture must not touch (memo, workspace, pinned pool)
         torch.cuda.synchronize()
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph):
             cur = torch.cuda.current_stream()
             ready = torch.cuda.Event()
             ready.record(cur)
-            F = plan.synthesize(data, t)
+            F = plan.synthesize(data, t, companions=companions)
             self.prep = plan.prepare(t, overlapped=True, after=ready, speculate=True)
             if self.prep._assumed is None:
                 raise RuntimeError("CapturedTransform: the time axis must have been prepared once before the capture")
@@ -875,11 +933,13 @@ class CapturedTransform:
         return (lo, hi) == tuple(self.prep._assumed[:2])
 
 
-def _capture(self, t, data):
-    """See CapturedTransform."""
-    if self.mix:
-        raise NotImplementedError("capture does not cover psi0..psi3 (their companion fields are uploaded per call)")
-    return CapturedTransform(self, t, data)
+def _capture(self, t, data, companions=None):
+    """See CapturedTransform.  psi0..psi3 need `companions` (device tensors, as for `run`): a graph cannot contain the
+    upload of the psi*_modes the plan was built with."""
+    if self.mix and companions is None:
+        raise ValueError("capture of psi0..psi3 needs companions=[psi(n+1), ..., psi4] as device tensors")
+    self._check_companions(companions, (data.shape[0],))
+    return CapturedTransform(self, t, data, companions)
 
 
 TransformPlan.capture = _capture
@@ -967,20 +1027,26 @@ def cached_transform_plan(ell_min, ell_max, dataType, r_is_scaled_out=True, out_
     return plan
 
 
-def _run_batch(self, t, data_batch, prep=None):
+def _run_batch(self, t, data_batch, prep=None, companions=None):
     """A batch of waveforms sharing the time axis and the transformation (BASELINE config 3): data_batch
     [B, N, n_modes] device tensor -> (u' [N'], modes' [B, N', n_modes_out]).  One synthesis launch over all B*N rows,
-    one spline launch with the batch in gridDim.z, one analysis launch over all B*N' rows."""
+    one spline launch with the batch in gridDim.z, one analysis launch over all B*N' rows.  psi0..psi3 need `companions`:
+    each waveform's higher Weyl scalars as [B, N, n_modes_q] complex128 device tensors ordered psi(n+1)..psi4 (layout of
+    the psi*_modes the plan was built with); each is synthesized over all B*N rows and one scrib200_weyl_mix_series launch
+    mixes the batch."""
     torch = self.torch
     B, N = int(data_batch.shape[0]), int(data_batch.shape[1])
     if t.shape[0] != N:
         raise ValueError("run_batch: the time axis must match dimension 1 of the batch")
-    if self.mix:
-        raise NotImplementedError("run_batch does not cover psi0..psi3 (they need their companion fields per waveform)")
+    if self.mix and companions is None:
+        raise ValueError("run_batch of psi0..psi3 needs companions=[psi(n+1), ..., psi4] as [B, N, n_modes] device tensors")
+    comps = self._check_companions(companions, (B, N))
+    if comps is not None:
+        comps = [c.reshape(B * N, -1) for c in comps]
     cur = torch.cuda.current_stream()
     ready = torch.cuda.Event()
     ready.record(cur)
-    F = self.synthesize(data_batch.reshape(B * N, -1))
+    F = self._synthesize(data_batch.reshape(B * N, -1), t, None, comps, B)
     mine = prep is None
     for attempt in range(2):
         if mine:
