@@ -500,13 +500,13 @@ def transform(abd, **kwargs):
         one_over_k = gamma * (1 - v_dot_r)
         k = 1.0 / one_over_k
         ethk_over_k = eth_v_dot_r / (1 - v_dot_r)
-        plan = GridPlan()
-        plan.divide_by_gamma = True    # transformations.py:393: timeprime = (u - alpha_00/sqrt(4 pi)) / gamma
-        plan._init_grid("cuda", n_theta, n_phi, gamma, (supertranslation[0] / math.sqrt(4 * math.pi)).real, k, alpha)
+        # transformations.py:393: timeprime = (u - alpha_00/sqrt(4 pi)) / gamma
+        plan = GridPlan("cuda", n_theta, n_phi, gamma, (supertranslation[0] / math.sqrt(4 * math.pi)).real, k, alpha, divide_by_gamma=True)
         dev = plan.device
         # the synthesis operands sY_lm(R_g) of the six spins are built and packed on the device (scrib200_swsh_pack), as in
         # TransformPlan: at ell_max = 32 the host recurrence + packing took 4 s, the kernels of the whole transform 0.1 s
         packs = {}
+        analyses = {}
         n_all = (abd.ell_max + 1) ** 2
         Kpad = -(-2 * n_all // 16) * 16
         Ncpad = -(-2 * G // 64) * 64
@@ -522,6 +522,7 @@ def transform(abd, **kwargs):
                 "swsh_pack",
             )
             packs[name] = (dB, Kpad, Ncpad)
+            analyses[name] = ops.analysis(s, 0, Lout, n_theta, n_phi)
     f64 = torch.float64
     d_zero = torch.zeros(Ncpad, dtype=f64, device=dev)
     d_unit = torch.zeros(Ncpad, dtype=f64, device=dev)
@@ -558,17 +559,10 @@ def transform(abd, **kwargs):
     # the result lands field by field in ONE pinned host block (torch's caching host allocator reuses it between calls):
     # each D2H is a DMA at PCIe rate queued behind that field's analysis, with no second host copy
     raw_t = torch.empty((len(FIELDS), n_out, (Lout + 1) ** 2), dtype=torch.complex128, pin_memory=True)
-    tile = int(_lib.load().scrib200_map2salm_tile_size(n_theta, n_phi, 0, Lout)) if n_out > 0 else 0
     for name in FIELDS:
-        s = SPINS[name]
         if n_out == 0:
             break
-        if tile:
-            gridT = plan._remap(t_d, F[name], uprm, prep, tile)
-            modes = ops.map2salm_tiled_device(gridT, tile, n_out, s, Lout, n_theta, n_phi)
-        else:
-            grid = plan.remap(t_d, F[name], uprm, prep)
-            modes = ops.map2salm(grid, s, Lout, n_theta, n_phi, ell_min=0)
+        modes = plan.remap_analyze(t_d, F[name], uprm, prep, analyses[name])
         del F[name]
         raw_t[FIELDS.index(name)].copy_(modes, non_blocking=True)
     cur.synchronize()

@@ -5,6 +5,7 @@ Each function is the drop-in for one numba / third-party kernel the reference ca
 tensors (then nothing is copied and a CUDA tensor is returned), which is what bench.py's
 device-resident `value` uses.  No CPU fallback: without a CUDA device these raise Scrib200Error.
 """
+import collections
 import ctypes
 import math
 import os
@@ -366,13 +367,7 @@ def _separable_analysis_tables(s, ell_min, ell_max, n_theta, n_phi):
 
 
 def map2salm(grid, s, ell_max, n_theta=None, n_phi=None, ell_min=0, separable=None):
-    """spinsfast.map2salm replacement, batched over leading axes: [..., n_theta, n_phi] -> [..., n_modes].  From
-    ell_max = 16 up the analysis is separable on the tensor cores - the phi-DFT as a GEMM over the rows (time, ring), then the
-    theta quadrature per M (scrib200_theta_quad); below that the shared-memory kernels of scrib200_map2salm."""
-    from .plan import map2salm as _m2s
-
-    torch = _torch()
-    lib = _lib.load()
+    """spinsfast.map2salm replacement, batched over leading axes: [..., n_theta, n_phi] -> [..., n_modes] (see `analyze`)."""
     if is_tensor(grid):
         g = grid
     else:
@@ -381,16 +376,50 @@ def map2salm(grid, s, ell_max, n_theta=None, n_phi=None, ell_min=0, separable=No
         n_theta, n_phi = g.shape[-2:]
     lead = g.shape[:-2] if g.dim() >= 2 and g.shape[-2:] == (n_theta, n_phi) else g.shape[:-1]
     g2 = g.reshape(-1, n_theta * n_phi)
-    sep = _separable_analysis_tables(s, ell_min, ell_max, n_theta, n_phi) if (separable or (separable is None and ell_max >= 16)) else None
+    out = analyze(g2, analysis(s, ell_min, ell_max, n_theta, n_phi), separable).reshape(tuple(lead) + (-1,))
+    return out if is_tensor(grid) else to_host(out)
+
+
+Analysis = collections.namedtuple("Analysis", "s ell_min ell_max n_theta n_phi n_modes E Wt trig tile")
+_analysis_cache = {}
+
+
+def analysis(s, ell_min, ell_max, n_theta, n_phi):
+    """The SWSH analysis of spin `s` onto ell_min..ell_max from the n_theta x n_phi grid, cached per (spin, ell range, grid,
+    device): the tables E, Wt of scrib200_map2salm (scri_b200._sf.analysis_tables), `trig` = (cos, sin)(m phi_k)/n_phi for
+    m = 0..ell_max of scrib200_map2salm_tiled (the +m column of E is (cos - i sin)/n_phi), and the time tile of the tiled
+    kernel (scrib200_map2salm_tile_size; 0 when its tables do not fit: the time-major kernels then)."""
+    torch = _torch()
+    key = (s, ell_min, ell_max, n_theta, n_phi, torch.cuda.current_device())
+    if key not in _analysis_cache:
+        E, Wt = _sf.analysis_tables(s, ell_min, ell_max, n_theta, n_phi)
+        trig = np.conj(E[:, ell_max:])
+        E, Wt, trig = (torch.from_numpy(np.ascontiguousarray(x)).cuda() for x in (E, Wt, trig))
+        tile = int(_lib.load().scrib200_map2salm_tile_size(n_theta, n_phi, ell_min, ell_max))
+        _analysis_cache[key] = Analysis(s, ell_min, ell_max, n_theta, n_phi, _sf.LM_total_size(ell_min, ell_max), E, Wt, trig, tile)
+    return _analysis_cache[key]
+
+
+def analyze(grid, an, separable=None):
+    """Analysis `an` of a time-major device grid [N, n_theta * n_phi] complex128 -> [N, an.n_modes].  From ell_max = 16 up
+    it is separable on the tensor cores when its tables fit - the phi-DFT as a GEMM over the rows (time, ring), then the
+    theta quadrature per M (scrib200_theta_quad); otherwise the shared-memory kernels of scrib200_map2salm.  `separable`
+    True / False forces one path."""
+    torch = _torch()
+    lib = _lib.load()
+    n_theta, n_phi, ell_max = an.n_theta, an.n_phi, an.ell_max
+    sep = (_separable_analysis_tables(an.s, an.ell_min, ell_max, n_theta, n_phi)
+           if (separable or (separable is None and ell_max >= 16)) else None)
     if separable and sep is None:
         raise _lib.Scrib200Error("map2salm: the separable analysis tables do not fit at this ell_max")
+    N = grid.shape[0]
     if sep is not None:
         tb, dev, dB, Kpad, Ncpad, unit, zero = sep
-        N, nm = g2.shape[0], 2 * ell_max + 1
-        g2 = g2.contiguous()
+        nm = 2 * ell_max + 1
+        grid = grid.contiguous()
         P = torch.empty((N, n_theta, nm), dtype=torch.complex128, device="cuda")
         _lib.check(
-            lib.scrib200_swsh_synthesize(_lib.ptr(g2), N * n_theta, n_phi, _lib.ptr(dB), Kpad, Ncpad, _lib.ptr(zero), _lib.ptr(unit), nm,
+            lib.scrib200_swsh_synthesize(_lib.ptr(grid), N * n_theta, n_phi, _lib.ptr(dB), Kpad, Ncpad, _lib.ptr(zero), _lib.ptr(unit), nm,
                                          _lib.ptr(P), _lib.stream_ptr()),
             "swsh_synthesize(phi-DFT)",
         )
@@ -400,39 +429,16 @@ def map2salm(grid, s, ell_max, n_theta=None, n_phi=None, ell_min=0, separable=No
                                     tb.cfg.ctypes.data_as(ctypes.c_void_p), _lib.ptr(out), _lib.stream_ptr()),
             "theta_quad",
         )
-        out = out.reshape(tuple(lead) + (-1,))
-        return out if is_tensor(grid) else to_host(out)
-    E, Wt = _sf.analysis_tables(s, ell_min, ell_max, n_theta, n_phi)
-    dE = torch.from_numpy(np.ascontiguousarray(E)).cuda()
-    dW = torch.from_numpy(Wt).cuda()
-    out = _m2s(g2, n_theta, n_phi, ell_min, ell_max, dE, dW).reshape(tuple(lead) + (-1,))
-    return out if is_tensor(grid) else to_host(out)
-
-
-_analysis_cache = {}
-
-
-def _analysis_device_tables(s, ell_min, ell_max, n_theta, n_phi):
-    """(E, Wt, trig) of scri_b200._sf.analysis_tables on the current device, cached per (spin, ell range, grid)."""
-    torch = _torch()
-    key = (s, ell_min, ell_max, n_theta, n_phi, torch.cuda.current_device())
-    if key not in _analysis_cache:
-        E, Wt = _sf.analysis_tables(s, ell_min, ell_max, n_theta, n_phi)
-        trig = np.ascontiguousarray(np.conj(E[:, ell_max:]))
-        _analysis_cache[key] = tuple(torch.from_numpy(np.ascontiguousarray(x)).cuda() for x in (E, Wt, trig))
-    return _analysis_cache[key]
-
-
-def map2salm_tiled_device(gridT, tile, n_out, s, ell_max, n_theta, n_phi, ell_min=0):
-    """Analysis of a time-tiled device grid [ceil(n_out/tile), G, tile] (the layout scrib200_spline_remap writes)."""
-    torch = _torch()
-    lib = _lib.load()
-    _, dW, dtrig = _analysis_device_tables(s, ell_min, ell_max, n_theta, n_phi)
-    out = torch.empty((n_out, _sf.LM_total_size(ell_min, ell_max)), dtype=torch.complex128, device="cuda")
+        return out
+    out = torch.empty((N, an.n_modes), dtype=torch.complex128, device=grid.device)
+    need = lib.scrib200_map2salm_workspace_bytes(N, n_theta, n_phi, ell_max)
+    ws = torch.empty(max(need, 16), dtype=torch.uint8, device=grid.device)
     _lib.check(
-        lib.scrib200_map2salm_tiled(_lib.ptr(gridT), tile, n_out, n_theta, n_phi, _lib.ptr(dtrig), _lib.ptr(dW), ell_min, ell_max,
-                                    _lib.ptr(out), _lib.stream_ptr()),
-        "map2salm_tiled",
+        lib.scrib200_map2salm(
+            _lib.ptr(grid), N, n_theta, n_phi, _lib.ptr(an.E), _lib.ptr(an.Wt), an.ell_min, ell_max, _lib.ptr(out),
+            _lib.ptr(ws), ws.numel(), _lib.stream_ptr(),
+        ),
+        "map2salm",
     )
     return out
 

@@ -336,8 +336,4 @@ def sharded_transform(plan, t_local, data_local, companions_local=None, halo=Non
     if n_out == 0:
         return uprm, torch.empty((0, plan.n_modes_out), dtype=torch.complex128, device=dev)
     torch.cuda.current_stream().wait_event(prep.done)
-    if plan.tile:
-        modes = plan.analyze_tiled(plan._remap(t_ext, F, uprm, prep, plan.tile), n_out)
-    else:
-        modes = plan.analyze(plan.remap(t_ext, F, uprm, prep))
-    return uprm, modes
+    return uprm, plan.remap_analyze(t_ext, F, uprm, prep, plan.analysis)

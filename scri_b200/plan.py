@@ -224,11 +224,11 @@ def _quiet_blas():
 
 class GridPlan:
     """What every transformation shares once the rotor grid is fixed: the conformal factor and supertranslation on the
-    grid (device arrays `d_k`, `d_alpha`), the output time axis, and the spline remap / analysis launches."""
+    grid (device arrays `d_k`, `d_alpha`), the output time axis, and the synthesis, spline remap and analysis launches.
+    `divide_by_gamma`: u' = (t - dt) / gamma as the ABD path forms it (transformations.py:393); otherwise
+    u' = (1/gamma)(t - dt) as in waveform_grid.py:565."""
 
-    divide_by_gamma = False   # u' = (1/gamma)(t - dt) as in waveform_grid.py:565; the ABD path divides by gamma instead
-
-    def _init_grid(self, device, n_theta, n_phi, gamma, time_translation, kconformal, alpha):
+    def __init__(self, device, n_theta, n_phi, gamma, time_translation, kconformal, alpha, divide_by_gamma=False):
         torch = _lib.require_cuda()
         _lib.load()
         self.torch = torch
@@ -237,6 +237,7 @@ class GridPlan:
         self.G = self.n_theta * self.n_phi
         self.gamma = gamma
         self.time_translation = time_translation
+        self.divide_by_gamma = divide_by_gamma
         self.kconformal, self.alpha = kconformal, alpha
         self.d_k = torch.from_numpy(np.ascontiguousarray(kconformal)).to(self.device)
         self.d_alpha = torch.from_numpy(np.ascontiguousarray(alpha)).to(self.device)
@@ -344,36 +345,81 @@ class GridPlan:
         """Spline each grid point's series from knots k(t-alpha) onto u' (waveform_grid.py:576-588); [N', G]."""
         return self._remap(t, F, uprm, prep, 0)
 
-    def synthesize_with(self, data, d_B, n_modes, Kpad, Ncpad, d_offset, d_scale):
-        """Synthesis of one field against its own packed table: [N, n_modes] complex128 -> [N, G].  The table is re-laid out
-        as three real planes (one pass over it, ~0.3 ms at ell_max = 32) and the three-multiplication kernel does the product:
-        the ABD synthesis sits on the FP64 tensor pipe (92 % DMMA activity in round 1), where 6 n G flops instead of 8 n G
-        is a quarter of the time; SCRIB200_SYNTH_FOLDED keeps the one-GEMM form."""
+    def synthesize_with(self, data, d_B, n_modes, Kpad, Ncpad, d_offset, d_scale, out=None, d_B3=None, folded=False):
+        """Synthesis of `data` [rows, n_modes] complex128 against the packed table `d_B` (pack_synthesis_matrix layout), one
+        launch into `out` [rows, G] (allocated when None).  By default the three-multiplication kernel on the table's three
+        real planes Y_r, Y_i, Y_r + Y_i: `d_B3` when the caller keeps them, else packed here (one pass over the table,
+        ~0.3 ms at ell_max = 32) and freed after, so that fields synthesized one after the other never hold two sets.  On the
+        FP64 tensor pipe (92 % DMMA activity in round 1) 6 n G flops instead of 8 n G is a quarter of the time.  `folded`,
+        or SCRIB200_SYNTH_FOLDED set, takes the one-GEMM form instead; the two round differently, so each caller keeps
+        the kernel it has."""
         import os
 
         torch = self.torch
-        N = data.shape[0]
-        F = torch.empty((N, self.G), dtype=torch.complex128, device=self.device)
-        if not os.environ.get("SCRIB200_SYNTH_FOLDED"):
-            lib = _lib.load()
-            npad3, Gpad3 = -(-n_modes // 8) * 8, -(-self.G // 32) * 32
+        lib = _lib.load()
+        rows = data.shape[0]
+        if out is None:
+            out = torch.empty((rows, self.G), dtype=torch.complex128, device=self.device)
+        if folded or os.environ.get("SCRIB200_SYNTH_FOLDED"):
+            _lib.check(
+                lib.scrib200_swsh_synthesize(
+                    _lib.ptr(data), rows, n_modes, _lib.ptr(d_B), Kpad, Ncpad, _lib.ptr(d_offset), _lib.ptr(d_scale), self.G,
+                    _lib.ptr(out), _lib.stream_ptr(),
+                ),
+                "swsh_synthesize",
+            )
+            return out
+        npad3, Gpad3 = -(-n_modes // 8) * 8, -(-self.G // 32) * 32
+        if d_B3 is None:
             d_B3 = torch.empty((3, npad3, Gpad3), dtype=torch.float64, device=self.device)
             _lib.check(lib.scrib200_swsh_pack3m(_lib.ptr(d_B), Kpad, Ncpad, n_modes, self.G, _lib.ptr(d_B3), npad3, Gpad3, _lib.stream_ptr()),
                        "swsh_pack3m")
-            _lib.check(
-                lib.scrib200_swsh_synthesize_3m(_lib.ptr(data), N, n_modes, _lib.ptr(d_B3), npad3, Gpad3, _lib.ptr(d_offset), _lib.ptr(d_scale),
-                                                self.G, _lib.ptr(F), _lib.stream_ptr()),
-                "swsh_synthesize_3m",
-            )
-            return F
         _lib.check(
-            _lib.load().scrib200_swsh_synthesize(
-                _lib.ptr(data), N, n_modes, _lib.ptr(d_B), Kpad, Ncpad, _lib.ptr(d_offset), _lib.ptr(d_scale), self.G,
-                _lib.ptr(F), _lib.stream_ptr(),
-            ),
-            "swsh_synthesize",
+            lib.scrib200_swsh_synthesize_3m(_lib.ptr(data), rows, n_modes, _lib.ptr(d_B3), npad3, Gpad3, _lib.ptr(d_offset), _lib.ptr(d_scale),
+                                            self.G, _lib.ptr(out), _lib.stream_ptr()),
+            "swsh_synthesize_3m",
         )
-        return F
+        return out
+
+    def analyze(self, grid, analysis=None):
+        """[N', G] complex128, time-major -> [N', n_modes_out] (waveform_grid.py:303-307) by `analysis` (ops.analysis;
+        default the plan's own): large band limits take the separable tensor-core analysis, the rest the shared-memory
+        kernels (ops.analyze)."""
+        from . import ops
+
+        an = analysis or self.analysis
+        if grid.shape[0] == 0:
+            return self.torch.empty((0, an.n_modes), dtype=self.torch.complex128, device=self.device)
+        return ops.analyze(grid, an)
+
+    def analyze_tiled(self, gridT, n_out, out=None, analysis=None):
+        """gridT [ceil(n_out/T), G, T] complex128 (time-tiled, T = the analysis' tile) -> [n_out, n_modes_out]."""
+        an = analysis or self.analysis
+        torch = self.torch
+        if out is None:
+            out = torch.empty((n_out, an.n_modes), dtype=torch.complex128, device=self.device)
+        if n_out == 0:
+            return out
+        _lib.check(
+            _lib.load().scrib200_map2salm_tiled(
+                _lib.ptr(gridT), an.tile, n_out, self.n_theta, self.n_phi, _lib.ptr(an.trig), _lib.ptr(an.Wt), an.ell_min, an.ell_max,
+                _lib.ptr(out), _lib.stream_ptr(),
+            ),
+            "map2salm_tiled",
+        )
+        return out
+
+    def remap_analyze(self, t, F, uprm, prep, analysis, n_series=1, rows_needed=None, grid_out=None, out=None):
+        """Spline remap of F [n_series * N, G] onto u' and the analysis `analysis` (ops.analysis) of the result:
+        [n_series * N', n_modes].  The remapped grid is handed over time-tiled (scrib200_spline_remap with the analysis'
+        tile, then scrib200_map2salm_tiled) when the analysis has a tile, time-major (`remap`, `analyze`) when its tables
+        are too large for that.  `rows_needed` as for `_remap`; `grid_out` and `out` are caller buffers for the tiled
+        grid and the modes of the tiled path."""
+        n_out = n_series * uprm.shape[0]
+        grid = self._remap(t, F, uprm, prep, analysis.tile, n_series, rows_needed, grid_out)
+        if analysis.tile:
+            return self.analyze_tiled(grid, n_out, out, analysis)
+        return self.analyze(grid, analysis)
 
     def weyl_mix(self, fields, coefs, t, d_A, d_C, d_scale, d_offset, out):
         """One scrib200_weyl_mix launch (see include/scrib200.h)."""
@@ -403,10 +449,6 @@ class TransformPlan(GridPlan):
             self._build(ell_min, ell_max, dataType, r_is_scaled_out, out_ell_max, device, kwargs)
 
     def _build(self, ell_min, ell_max, dataType, r_is_scaled_out, out_ell_max, device, kwargs):
-        torch = _lib.require_cuda()
-        _lib.load()
-        self.torch = torch
-        self.device = torch.device(device)
         self.ell_min, self.ell_max, self.dataType = int(ell_min), int(ell_max), int(dataType)
         self.spin_weight = SpinWeights[self.dataType]
         self.conformal_weight = ConformalWeights[self.dataType] - (RScaling[self.dataType] if r_is_scaled_out else 0)
@@ -426,9 +468,7 @@ class TransformPlan(GridPlan):
         ) = process_transformation_kwargs(self.ell_max, **kwargs)
         self.leftover_kwargs = leftover
         self.supertranslation = supertranslation
-        self.L, self.n_theta, self.n_phi = L, n_theta, n_phi
-        self.G = n_theta * n_phi
-        self.gamma, self.beta = gamma, beta
+        self.L, self.beta = L, beta
         self.out_ell_max = self.ell_max if out_ell_max is None else int(out_ell_max)
         self.out_ell_min = abs(self.spin_weight)
         s = self.spin_weight
@@ -439,8 +479,10 @@ class TransformPlan(GridPlan):
         Y = _sf.SWSH_grid(R, s, ell_max_st) if self.dataType in (h, sigma) else None
         SH = _sf.SWSH_grid(R, 0, ell_max_st)
         rhat = Q.rotate_z(R)
-        self.kconformal = 1.0 / (gamma * (1 - rhat @ boost_velocity))
-        self.alpha = (SH @ supertranslation).real
+        kconformal = 1.0 / (gamma * (1 - rhat @ boost_velocity))
+        super().__init__(device, n_theta, n_phi, gamma, (supertranslation[0] / math.sqrt(4 * math.pi)).real, kconformal,
+                         (SH @ supertranslation).real)
+        torch = self.torch
         offset_c = np.zeros(self.G, dtype=complex)
         self.mix = []          # higher Weyl scalars mixed into psi0..psi3 (empty for every other data type)
         nontrivial = beta != 0 or (supertranslation[1:] != 0).any()
@@ -500,8 +542,6 @@ class TransformPlan(GridPlan):
         scl = np.zeros(self.Ncpad)
         scl[0 : 2 * self.G : 2] = 1.0 if self.mix else scale     # with mixing the weight k^w is applied after the sum
         scl[1 : 2 * self.G : 2] = 1.0 if self.mix else scale
-        self.time_translation = (supertranslation[0] / math.sqrt(4 * math.pi)).real
-        E, Wt = _sf.analysis_tables(s, self.out_ell_min, self.out_ell_max, n_theta, n_phi)
         self.n_modes_in = _sf.LM_total_size(self.ell_min, self.ell_max)
         self.n_modes_out = _sf.LM_total_size(self.out_ell_min, self.out_ell_max)
 
@@ -538,44 +578,8 @@ class TransformPlan(GridPlan):
             self.d_mixA = torch.from_numpy(np.ascontiguousarray(self.mix_A)).to(dev)
             self.d_mixC = torch.from_numpy(np.ascontiguousarray(self.mix_C)).to(dev)
             self.d_mixscale = torch.from_numpy(np.ascontiguousarray(scale)).to(dev)
-        self.d_k = torch.from_numpy(np.ascontiguousarray(self.kconformal)).to(dev)
-        self.d_alpha = torch.from_numpy(np.ascontiguousarray(self.alpha)).to(dev)
-        self.d_E = torch.from_numpy(np.ascontiguousarray(E)).to(dev)
-        self.d_Wt = torch.from_numpy(Wt).to(dev)
-        # (cos, sin)(m phi_k)/n_phi for m = 0..L: the +m column of E is (cos - i sin)/n_phi
-        Lo = self.out_ell_max
-        trig = np.ascontiguousarray(np.conj(E[:, Lo:]))
-        self.d_trig = torch.from_numpy(trig).to(dev)
-        self._tile = None
-        self._ws = None
-        self._d2h_stream = None
-        self._side = None
-        self._host_pool = []
-        self.spline_halo = 0   # 0 = chosen from the decay diagnostics of scrib200_spline_prepare
-        self.spline_body = 0   # 0 = default intervals per tile
-
-    def _synthesize_rows(self, data, F):
-        """F[rows] = synthesis of data[rows] (one launch): the three-multiplication kernel, or the folded real GEMM with
-        SCRIB200_SYNTH_FOLDED set."""
-        import os
-
-        lib = _lib.load()
-        if os.environ.get("SCRIB200_SYNTH_FOLDED"):
-            _lib.check(
-                lib.scrib200_swsh_synthesize(
-                    _lib.ptr(data), data.shape[0], self.n_modes_in, _lib.ptr(self.d_B), self.Kpad, self.Ncpad,
-                    _lib.ptr(self.d_offset), _lib.ptr(self.d_scale), self.G, _lib.ptr(F), _lib.stream_ptr(),
-                ),
-                "swsh_synthesize",
-            )
-        else:
-            _lib.check(
-                lib.scrib200_swsh_synthesize_3m(
-                    _lib.ptr(data), data.shape[0], self.n_modes_in, _lib.ptr(self.d_B3), self.npad3, self.Gpad3,
-                    _lib.ptr(self.d_offset), _lib.ptr(self.d_scale), self.G, _lib.ptr(F), _lib.stream_ptr(),
-                ),
-                "swsh_synthesize_3m",
-            )
+        with torch.cuda.device(dev):
+            self.analysis = ops.analysis(s, self.out_ell_min, self.out_ell_max, n_theta, n_phi)
 
     def _check_companions(self, companions, rows, host=False):
         """Check the companion fields of psi0..psi3 passed to one call: a list or tuple ordered psi(n+1)..psi4, each of
@@ -624,16 +628,21 @@ class TransformPlan(GridPlan):
         comps = self._check_companions(companions, (N,))
         if self.mix and t is None:
             raise ValueError("TransformPlan.synthesize needs the time axis for psi0..psi3")
-        if self.mix and comps is None:
-            from . import ops
+        return self._synthesize(data, t, slabs, self._planned_companions(N) if comps is None else comps, 1)
 
-            comps = []
-            for mx in self.mix:
-                d = ops.to_device(mx["data"], np.complex128)
-                if d.shape[0] != N:
-                    raise ValueError("psi*_modes must share the time axis of the waveform being transformed")
-                comps.append(d)
-        return self._synthesize(data, t, slabs, comps, 1)
+    def _planned_companions(self, N):
+        """The psi*_modes the plan was built with as device tensors (None for a plan that mixes in none)."""
+        from . import ops
+
+        if not self.mix:
+            return None
+        comps = []
+        for mx in self.mix:
+            d = ops.to_device(mx["data"], np.complex128)
+            if d.shape[0] != N:
+                raise ValueError("psi*_modes must share the time axis of the waveform being transformed")
+            comps.append(d)
+        return comps
 
     def _synthesize(self, data, t, slabs, comps, n_series):
         """Synthesis of `data` [n_series * N, n_modes] (series stacked along time), then for psi0..psi3 the synthesis of each
@@ -652,20 +661,14 @@ class TransformPlan(GridPlan):
                 cur.wait_event(ev)
             if hi <= lo:
                 continue
-            self._synthesize_rows(data[lo:hi], F[lo:hi])
+            self.synthesize_with(data[lo:hi], self.d_B, self.n_modes_in, self.Kpad, self.Ncpad, self.d_offset, self.d_scale,
+                                 out=F[lo:hi], d_B3=self.d_B3)
         if not self.mix:
             return F
         fields, coefs = [F], [1.0]
         for mx, d in zip(self.mix, comps):
-            Fq = torch.empty((rows, self.G), dtype=torch.complex128, device=self.device)
-            _lib.check(
-                lib.scrib200_swsh_synthesize(
-                    _lib.ptr(d), rows, mx["n_modes"], _lib.ptr(mx["d_B"]), mx["Kpad"], mx["Ncpad"], _lib.ptr(self.d_zero),
-                    _lib.ptr(self.d_unit), self.G, _lib.ptr(Fq), _lib.stream_ptr(),
-                ),
-                "swsh_synthesize",
-            )
-            fields.append(Fq)
+            fields.append(self.synthesize_with(d, mx["d_B"], mx["n_modes"], mx["Kpad"], mx["Ncpad"], self.d_zero, self.d_unit,
+                                               folded=True))
             coefs.append(mx["coef"])
         ptrs = (ctypes.c_void_p * len(fields))(*[f.data_ptr() for f in fields])
         cf = (ctypes.c_double * len(coefs))(*coefs)
@@ -678,47 +681,15 @@ class TransformPlan(GridPlan):
         )
         return F
 
-    def analyze(self, grid):
-        """[N', G] complex128 -> [N', n_modes_out] (waveform_grid.py:303-307).  Large band limits take the separable
-        tensor-core analysis (phi-DFT GEMM + scrib200_theta_quad), the rest the shared-memory kernels."""
-        if grid.shape[0] == 0:
-            return self.torch.empty((0, self.n_modes_out), dtype=self.torch.complex128, device=self.device)
-        if self.out_ell_max >= 16:
-            from . import ops
-
-            if ops._separable_analysis_tables(self.spin_weight, self.out_ell_min, self.out_ell_max, self.n_theta, self.n_phi) is not None:
-                return ops.map2salm(grid.reshape(-1, self.n_theta, self.n_phi), self.spin_weight, self.out_ell_max, self.n_theta, self.n_phi,
-                                    ell_min=self.out_ell_min, separable=True)
-        return map2salm(grid, self.n_theta, self.n_phi, self.out_ell_min, self.out_ell_max, self.d_E, self.d_Wt)
-
-    # -- time-tiled variants: the layout the fused transform path uses between remap and analysis ----
+    # -- time-tiled remap: the layout the fused transform path hands from the remap to the analysis
     def remap_tiled(self, t, F, uprm, prep=None):
         """Same spline remap, result stored time-tiled: [ceil(N'/T), G, T] (T = self.tile)."""
         return self._remap(t, F, uprm, prep, self.tile)
 
-    def analyze_tiled(self, gridT, n_out, out=None):
-        """gridT [ceil(N'/T), G, T] complex128 (time-tiled) -> [n_out, n_modes_out]."""
-        torch = self.torch
-        lib = _lib.load()
-        if out is None:
-            out = torch.empty((n_out, self.n_modes_out), dtype=torch.complex128, device=self.device)
-        if n_out == 0:
-            return out
-        _lib.check(
-            lib.scrib200_map2salm_tiled(
-                _lib.ptr(gridT), self.tile, n_out, self.n_theta, self.n_phi, _lib.ptr(self.d_trig), _lib.ptr(self.d_Wt),
-                self.out_ell_min, self.out_ell_max, _lib.ptr(out), _lib.stream_ptr(),
-            ),
-            "map2salm_tiled",
-        )
-        return out
-
     @property
     def tile(self):
         """Time-tile size of the remap -> analysis hand-off (0: tables too large, use the time-major kernels)."""
-        if self._tile is None:
-            self._tile = int(_lib.load().scrib200_map2salm_tile_size(self.n_theta, self.n_phi, self.out_ell_min, self.out_ell_max))
-        return self._tile
+        return self.analysis.tile
 
     def _remap_analyze_to_host(self, t, F, uprm, prep, n_slabs):
         """Spline remap + analysis per slab of OUTPUT times, each slab's modes copied to pinned host memory on a copy stream
@@ -731,20 +702,18 @@ class TransformPlan(GridPlan):
         if self._d2h_stream is None:
             self._d2h_stream = torch.cuda.Stream()
         cs = self._d2h_stream
-        tile = self.tile
         per = -(-n_out // n_slabs)
-        per = -(-per // tile) * tile
+        per = -(-per // self.tile) * self.tile
         for lo in range(0, n_out, per):
             hi = min(n_out, lo + per)
-            gridT = self._remap(t, F, uprm[lo:hi], prep, tile)
-            modes = self.analyze_tiled(gridT, hi - lo)
+            modes = self.remap_analyze(t, F, uprm[lo:hi], prep, self.analysis)
             done = torch.cuda.Event()
             done.record(cur)
             cs.wait_event(done)
             with torch.cuda.stream(cs):
                 host[lo:hi].copy_(modes, non_blocking=True)
             modes.record_stream(cs)
-            del gridT, modes
+            del modes
         cs.synchronize()
         return host.numpy()
 
@@ -811,13 +780,13 @@ class TransformPlan(GridPlan):
             _trace(f"slab {k} queued on the copy stream")
             cur.wait_event(ev)
             if rhi > rlo:
-                self._synthesize_rows(data[rlo:rhi], F[rlo:rhi])
+                self.synthesize_with(data[rlo:rhi], self.d_B, self.n_modes_in, self.Kpad, self.Ncpad, self.d_offset, self.d_scale,
+                                     out=F[rlo:rhi], d_B3=self.d_B3)
             out_hi = n_out if k == len(slabs) - 1 else min(n_out, max(done, ((rhi - margin - lo) // tile) * tile))
             if out_hi > done:
                 rows_needed = self.input_rows_for_outputs(t_host, u_of_row(lo + done), u_of_row(lo + out_hi - 1))
-                gridT = self._remap(t, F, uprm[done:out_hi], prep, tile, rows_needed=rows_needed,
-                                    out=gridT_all[: -(-(out_hi - done) // tile)])
-                modes = self.analyze_tiled(gridT, out_hi - done, out=modes_all[done:out_hi])
+                modes = self.remap_analyze(t, F, uprm[done:out_hi], prep, self.analysis, rows_needed=rows_needed,
+                                           grid_out=gridT_all[: -(-(out_hi - done) // tile)], out=modes_all[done:out_hi])
                 ready = torch.cuda.Event(enable_timing=timing is not None)
                 ready.record(cur)
                 cs.wait_event(ready)
@@ -854,35 +823,76 @@ class TransformPlan(GridPlan):
         (the end-to-end path of WaveformGrid.transform).  `companions` (psi0..psi3 only): this waveform's higher Weyl
         scalars as [N, n_modes_q] complex128 device tensors ordered psi(n+1)..psi4, in the layout of the psi*_modes the plan
         was built with; None uses those psi*_modes themselves."""
-        self._check_companions(companions, (data.shape[0],))
+        comps = self._check_companions(companions, (data.shape[0],))
         if host_slabs and slabs is not None and t_host is not None and prep is None and self.tile and not self.mix and not return_grid:
             streamed = self._run_streaming(t, data, slabs, t_host, on_queued=on_queued)
             if streamed is not None:
                 return streamed
-        cur = self.torch.cuda.current_stream()
-        ready = self.torch.cuda.Event()
+        comps = self._planned_companions(data.shape[0]) if comps is None else comps
+
+        def finish(F, uprm, prep):
+            if return_grid:
+                return self.remap(t, F, uprm, prep)
+            if host_slabs and self.tile and uprm.shape[0] >= 8192:
+                return self._remap_analyze_to_host(t, F, uprm, prep, host_slabs)
+            return self.remap_analyze(t, F, uprm, prep, self.analysis)
+
+        prep, out = self._step(t, data, comps, slabs=slabs, prep=prep, finish=finish)
+        return prep.uprm, out
+
+    def run_batch(self, t, data_batch, prep=None, companions=None):
+        """A batch of waveforms sharing the time axis and the transformation (BASELINE config 3): data_batch
+        [B, N, n_modes] device tensor -> (u' [N'], modes' [B, N', n_modes_out]).  One synthesis launch over all B*N rows,
+        one spline launch with the batch in gridDim.z, one analysis launch over all B*N' rows.  psi0..psi3 need `companions`:
+        each waveform's higher Weyl scalars as [B, N, n_modes_q] complex128 device tensors ordered psi(n+1)..psi4 (layout of
+        the psi*_modes the plan was built with); each is synthesized over all B*N rows and one scrib200_weyl_mix_series launch
+        mixes the batch."""
+        B, N = int(data_batch.shape[0]), int(data_batch.shape[1])
+        if t.shape[0] != N:
+            raise ValueError("run_batch: the time axis must match dimension 1 of the batch")
+        if self.mix and companions is None:
+            raise ValueError("run_batch of psi0..psi3 needs companions=[psi(n+1), ..., psi4] as [B, N, n_modes] device tensors")
+        comps = self._check_companions(companions, (B, N))
+        if comps is not None:
+            comps = [c.reshape(B * N, -1) for c in comps]
+        prep, modes = self._step(t, data_batch.reshape(B * N, -1), comps, n_series=B, prep=prep)
+        uprm = prep.uprm
+        return uprm, modes.reshape(B, uprm.shape[0], -1)
+
+    def capture(self, t, data, companions=None):
+        """See CapturedTransform.  psi0..psi3 need `companions` (device tensors, as for `run`): a graph cannot contain the
+        upload of the psi*_modes the plan was built with."""
+        if self.mix and companions is None:
+            raise ValueError("capture of psi0..psi3 needs companions=[psi(n+1), ..., psi4] as device tensors")
+        self._check_companions(companions, (data.shape[0],))
+        return CapturedTransform(self, t, data, companions)
+
+    def _step(self, t, data, comps, n_series=1, slabs=None, prep=None, finish=None, capturing=False):
+        """Queue one transform of `data` [n_series * N, n_modes] (series stacked along time; `slabs` as for `synthesize`)
+        mixed with the psi0..psi3 companions `comps` (same stacking): the synthesis, then - unless `prep` is given - the
+        preparation of `t` on the side stream under it, then `finish(F, uprm, prep)`, by default `remap_analyze`.  Returns
+        (prep, out).  A time axis seen before is prepared speculatively: its retained block is assumed, so the host does
+        not wait for the preparation kernels in the middle of the step (a caller streaming sub-batches would otherwise
+        drain its pipeline at every one); in the rare case the kernels found another block the step is queued once more,
+        unassumed.  `capturing` (a CUDA graph is being recorded): one attempt, the assumption required and verified by
+        the caller after a replay."""
+        torch = self.torch
+        cur = torch.cuda.current_stream()
+        ready = torch.cuda.Event()
         ready.record(cur)
-        F = self.synthesize(data, t, slabs, companions)     # queued first: the GPU is busy while the host launches the preparation
+        F = self._synthesize(data, t, slabs, comps, n_series)   # queued first: the GPU is busy while the host launches the preparation
         mine = prep is None
         for attempt in range(2):
             if mine:
-                # a time axis seen before: its retained block is assumed, so nothing waits for the read-back mid-step
                 prep = self.prepare(t, overlapped=True, after=ready, speculate=(attempt == 0))
+                if capturing and prep._assumed is None:
+                    raise RuntimeError("CapturedTransform: the time axis must have been prepared once before the capture")
             cur.wait_event(prep.done)
             uprm = prep.uprm
-            if self.tile and not return_grid:
-                if host_slabs and uprm.shape[0] >= 8192:
-                    out = self._remap_analyze_to_host(t, F, uprm, prep, host_slabs)
-                else:
-                    gridT = self.remap_tiled(t, F, uprm, prep)
-                    out = self.analyze_tiled(gridT, uprm.shape[0])
-                    del gridT
-            else:
-                grid = self.remap(t, F, uprm, prep)
-                out = grid if return_grid else self.analyze(grid)
-            if not mine or prep.verify():
-                return uprm, out
-            ready = self.torch.cuda.Event()       # the time axis changed behind the same storage: once more, unassumed
+            out = finish(F, uprm, prep) if finish else self.remap_analyze(t, F, uprm, prep, self.analysis, n_series)
+            if capturing or not mine or prep.verify():
+                return prep, out
+            ready = torch.cuda.Event()            # the time axis changed behind the same storage: once more, unassumed
             ready.record(cur)
 
 
@@ -901,22 +911,10 @@ class CapturedTransform:
         torch.cuda.synchronize()
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph):
-            cur = torch.cuda.current_stream()
-            ready = torch.cuda.Event()
-            ready.record(cur)
-            F = plan.synthesize(data, t, companions=companions)
-            self.prep = plan.prepare(t, overlapped=True, after=ready, speculate=True)
-            if self.prep._assumed is None:
-                raise RuntimeError("CapturedTransform: the time axis must have been prepared once before the capture")
-            cur.wait_event(self.prep.done)
+            self.prep, self.modes = plan._step(t, data, companions, capturing=True)
             self.uprm = self.prep.uprm
-            if plan.tile:
-                gridT = plan.remap_tiled(t, F, self.uprm, self.prep)
-                self.modes = plan.analyze_tiled(gridT, self.uprm.shape[0])
-            else:
-                self.modes = plan.analyze(plan.remap(t, F, self.uprm, self.prep))
             # the side stream (preparation + read-back of `info`) rejoins the capturing stream
-            cur.wait_stream(plan._side_stream())
+            torch.cuda.current_stream().wait_stream(plan._side_stream())
         self._info_host = self.prep._host                   # the graph's read-back lands here on every replay
         self.prep._host = None
 
@@ -931,18 +929,6 @@ class CapturedTransform:
         v = self._info_host.tolist()
         lo, hi = int(v[0]), max(int(v[0]), int(v[1]))
         return (lo, hi) == tuple(self.prep._assumed[:2])
-
-
-def _capture(self, t, data, companions=None):
-    """See CapturedTransform.  psi0..psi3 need `companions` (device tensors, as for `run`): a graph cannot contain the
-    upload of the psi*_modes the plan was built with."""
-    if self.mix and companions is None:
-        raise ValueError("capture of psi0..psi3 needs companions=[psi(n+1), ..., psi4] as device tensors")
-    self._check_companions(companions, (data.shape[0],))
-    return CapturedTransform(self, t, data, companions)
-
-
-TransformPlan.capture = _capture
 
 
 TRACE = None        # dev aid: set to a list to collect (label, perf_counter) marks of the end-to-end pipeline
@@ -1025,52 +1011,6 @@ def cached_transform_plan(ell_min, ell_max, dataType, r_is_scaled_out=True, out_
         while len(_plan_cache) > PLAN_CACHE_SIZE:
             _plan_cache.pop(next(iter(_plan_cache)))
     return plan
-
-
-def _run_batch(self, t, data_batch, prep=None, companions=None):
-    """A batch of waveforms sharing the time axis and the transformation (BASELINE config 3): data_batch
-    [B, N, n_modes] device tensor -> (u' [N'], modes' [B, N', n_modes_out]).  One synthesis launch over all B*N rows,
-    one spline launch with the batch in gridDim.z, one analysis launch over all B*N' rows.  psi0..psi3 need `companions`:
-    each waveform's higher Weyl scalars as [B, N, n_modes_q] complex128 device tensors ordered psi(n+1)..psi4 (layout of
-    the psi*_modes the plan was built with); each is synthesized over all B*N rows and one scrib200_weyl_mix_series launch
-    mixes the batch."""
-    torch = self.torch
-    B, N = int(data_batch.shape[0]), int(data_batch.shape[1])
-    if t.shape[0] != N:
-        raise ValueError("run_batch: the time axis must match dimension 1 of the batch")
-    if self.mix and companions is None:
-        raise ValueError("run_batch of psi0..psi3 needs companions=[psi(n+1), ..., psi4] as [B, N, n_modes] device tensors")
-    comps = self._check_companions(companions, (B, N))
-    if comps is not None:
-        comps = [c.reshape(B * N, -1) for c in comps]
-    cur = torch.cuda.current_stream()
-    ready = torch.cuda.Event()
-    ready.record(cur)
-    F = self._synthesize(data_batch.reshape(B * N, -1), t, None, comps, B)
-    mine = prep is None
-    for attempt in range(2):
-        if mine:
-            # a time axis seen before: its retained block is assumed, so the host does not wait for the preparation kernels
-            # in the middle of the call (a caller streaming sub-batches would otherwise drain its pipeline at every one)
-            prep = self.prepare(t, overlapped=True, after=ready, speculate=(attempt == 0))
-        cur.wait_event(prep.done)
-        uprm = prep.uprm
-        n_out = uprm.shape[0]
-        if self.tile:
-            gridT = self._remap(t, F, uprm, prep, self.tile, n_series=B)
-            modes = self.analyze_tiled(gridT, B * n_out)
-            del gridT
-        else:
-            grid = self._remap(t, F, uprm, prep, 0, n_series=B)
-            modes = self.analyze(grid)
-            del grid
-        if not mine or prep.verify():
-            return uprm, modes.reshape(B, n_out, -1)
-        ready = torch.cuda.Event()            # the time axis changed behind the same storage: once more, unassumed
-        ready.record(cur)
-
-
-TransformPlan.run_batch = _run_batch
 
 
 class TimePrep:
@@ -1170,22 +1110,3 @@ class TimePrep:
             d32, d64 = self._resolved[2:4]
             halo = 32 if d32 <= 1e-15 else (64 if d64 <= 1e-15 else 128)
         return int(halo), int(body)
-
-
-def map2salm(grid, n_theta, n_phi, ell_min, ell_max, d_E, d_Wt):
-    """Device map2salm: grid [N, n_theta*n_phi] complex128 -> [N, LM_total_size(ell_min, ell_max)]."""
-    torch = _lib.require_cuda()
-    lib = _lib.load()
-    N = grid.shape[0]
-    n_modes = _sf.LM_total_size(ell_min, ell_max)
-    out = torch.empty((N, n_modes), dtype=torch.complex128, device=grid.device)
-    need = lib.scrib200_map2salm_workspace_bytes(N, n_theta, n_phi, ell_max)
-    ws = torch.empty(max(need, 16), dtype=torch.uint8, device=grid.device)
-    _lib.check(
-        lib.scrib200_map2salm(
-            _lib.ptr(grid), N, n_theta, n_phi, _lib.ptr(d_E), _lib.ptr(d_Wt), ell_min, ell_max, _lib.ptr(out),
-            _lib.ptr(ws), ws.numel(), _lib.stream_ptr(),
-        ),
-        "map2salm",
-    )
-    return out
